@@ -10,6 +10,8 @@ controller with the viability-network terminal constraint, N=45, dt=5 ms, batch 
                                                             all host threads, bounded sample of the same workload)
   python bench.py --config cfg0|cfg1|cfg2|cfg3|cfg4 ...     the other BASELINE.json configurations (see PRESETS); the default and
                                                             the N = 1 headline stay cfg1
+  python bench.py ... --dump-outputs DIR                    also write what the last timed step computed as DIR/<name>.npy (see
+                                                            dump_outputs), so that two builds can be compared output for output
 """
 from __future__ import annotations
 
@@ -24,6 +26,7 @@ import numpy as np
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True      # the benchmark writes nothing into the tree it runs from (it may be read-only)
 
 from safe_mpc_b200 import abi, distributed as D  # noqa: E402
 from safe_mpc_b200.parser import Parameters, default_args  # noqa: E402
@@ -94,6 +97,33 @@ def warm_guess(main, x0, N, iters):
     main.reset_controller()
 
 
+DUMP_LIMIT = 64_000_000     # bytes --dump-outputs may write
+
+
+def dump_outputs(path, sim, main, step):
+    """What the closed loop hands its caller after `step` steps, as float64 .npy files under `path`: the plant state x [B, NX] after the
+    step and the control u [B, NU] applied in it, terminated [B] (1 for a problem whose simulation has ended, mpc.py's break: its log
+    rows are NaN, written here as zeros so that every output is finite), the main controller's warm start x_guess [B, N+1, NX] /
+    u_guess [B, N, NU] and its solve status [B].
+    When the batch would exceed DUMP_LIMIT, the same arrays for a fixed seeded sample of the problems; problem_index says which."""
+    x, u = sim.log()
+    x, u = x[:, step], u[:, step - 1]
+    terminated = np.isnan(x).any(axis=1) | np.isnan(u).any(axis=1)
+    xg, ug = main.get_guess()
+    out = {'x': np.where(terminated[:, None], 0.0, x), 'u': np.where(terminated[:, None], 0.0, u), 'terminated': terminated.astype(np.float64),
+           'x_guess': xg, 'u_guess': ug, 'status': main.get_state(abi.STATE_STATUS).astype(np.float64)}
+    B = main.B
+    per_problem = 8 * (1 + sum(v[0].size for v in out.values()))
+    idx = np.arange(B)
+    if B * per_problem > DUMP_LIMIT:
+        idx = np.sort(np.random.default_rng(0).choice(B, DUMP_LIMIT // per_problem, replace=False))
+    out = {k: np.ascontiguousarray(v[idx], dtype=np.float64) for k, v in out.items()}
+    out['problem_index'] = idx.astype(np.float64)
+    os.makedirs(path, exist_ok=True)
+    for k, v in out.items():
+        np.save(os.path.join(path, k + '.npy'), v)
+
+
 class ClockSampler:
     QUERY = ('index,clocks.sm,clocks.max.sm,power.draw,clocks_event_reasons.active,clocks_event_reasons.hw_slowdown,'
              'clocks_event_reasons.hw_thermal_slowdown,clocks_event_reasons.sw_thermal_slowdown,clocks_event_reasons.sw_power_cap')
@@ -130,8 +160,8 @@ class ClockSampler:
                 'reasons': sorted(reasons), 'samples': len(sm)}
 
 
-def time_oracle(controller, N, noise, seed, n_problems, steps, warmup, sqp_iters):
-    """The CPU path (oracle port of the reference's acados RTI path) on a bounded sample of the workload."""
+def time_oracle(controller, N, noise, seed, n_problems, steps, warmup, sqp_iters, dump=None):
+    """The CPU path (oracle port of the reference's acados RTI path) on a bounded sample of the workload; `dump`: dump_outputs directory."""
     from oracle.oracle import Oracle, OracleSim
     params, md, x0, pin = workload(controller, N, noise, seed, 0, n_problems)
     main, bk, prob = make_handles(Oracle, params, md, controller, n_problems, 0)
@@ -145,6 +175,8 @@ def time_oracle(controller, N, noise, seed, n_problems, steps, warmup, sqp_iters
     sim.run(steps)
     dt = time.perf_counter() - t0
     c1 = sim.counters()
+    if dump:
+        dump_outputs(dump, sim, main, warmup + steps)
     solves = (c1['rti_solves'] - c0['rti_solves']) + (c1['backup_solves'] - c0['backup_solves'])
     return {'value': solves / dt, 'seconds': dt, 'solves': solves, 'cores': main.num_threads(),
             'ipm_per_solve': (c1['ipm_iterations'] - c0['ipm_iterations']) / max(1, solves),
@@ -157,7 +189,7 @@ def run_reference(a):
     if rank != 0:
         return
     n = a.ref_problems
-    r = time_oracle(a.controller, a.horizon, a.noise, a.seed, n, a.steps, a.warmup, a.sqp_iters)
+    r = time_oracle(a.controller, a.horizon, a.noise, a.seed, n, a.steps, a.warmup, a.sqp_iters, dump=a.dump_outputs)
     line = {'metric': METRIC, 'value': r['value'], 'unit': UNIT, 'impl': 'reference', 'n_gpus': a.gpus, 'steps': a.steps, 'warmup': a.warmup,
             'ms_per_step': 1e3 * r['seconds'] / a.steps, 'higher_is_better': True, 'scaling': 'weak', 'vs_baseline': None, 'dtype': 'f64',
             'data': 'synthetic',
@@ -195,14 +227,18 @@ def run_engine(a):
     c0 = sim.counters(); l0 = main.launch_count() + bk.launch_count()
     D.barrier(); torch.cuda.synchronize()
     sampler = ClockSampler(local_rank) if rank == 0 else None
-    evs = [torch.cuda.Event(enable_timing=True) for _ in range(a.steps + 1)]
-    evs[0].record(stream)
-    for i in range(a.steps):
-        sim.step()
-        evs[i + 1].record(stream)
-    main.sync(); torch.cuda.synchronize()
-    D.barrier()
-    clocks = sampler.stop() if sampler else None
+    try:                                          # the sampler's nvidia-smi must not outlive a failed run
+        evs = [torch.cuda.Event(enable_timing=True) for _ in range(a.steps + 1)]
+        evs[0].record(stream)
+        for i in range(a.steps):
+            sim.step()
+            evs[i + 1].record(stream)
+        main.sync(); torch.cuda.synchronize()
+        D.barrier()
+    finally:
+        clocks = sampler.stop() if sampler else None
+    if a.dump_outputs:
+        dump_outputs(a.dump_outputs if world == 1 else os.path.join(a.dump_outputs, f'rank{rank}'), sim, main, a.warmup + a.steps)
     ms = evs[0].elapsed_time(evs[-1])
     lat = np.array([evs[i].elapsed_time(evs[i + 1]) for i in range(a.steps)])
     c1 = sim.counters(); l1 = main.launch_count() + bk.launch_count()
@@ -547,7 +583,12 @@ def main():
     ap.add_argument('--no-mlp', action='store_true', dest='no_mlp')
     ap.add_argument('--nn-precision', default=None, choices=['strict', 'tf32x3'], dest='nn_precision',
                     help='viability network arithmetic of the timed closed loop (the tensor-core kernel is always timed alone as well)')
+    ap.add_argument('--dump-outputs', default=None, metavar='DIR', dest='dump_outputs',
+                    help='after the timed steps, write what the last of them computed as DIR/<name>.npy (float64, at most 64 MB; '
+                         'with several GPUs DIR/rank<r>/)')
     a = ap.parse_args()
+    if a.steps < 1:
+        ap.error('--steps must be at least 1')
     pre = PRESETS[a.config]
     for key in ('controller', 'horizon', 'batch', 'noise'):
         if getattr(a, key) is None:

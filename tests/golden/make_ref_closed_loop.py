@@ -10,11 +10,13 @@ mpc.py is a flat script that builds acados solvers at its top; the statements of
   * ``model``          predicates, plant step and end-effector position evaluated by the oracle (bounds / collision checks, plant_step with
                        the nominal plant, kinematics), so that the scripted trajectories mean the same to both sides;
   * the remaining names (params, args, counters, ...) as plain values.
-Recorded: the x / u logs (NaN padded), conv / collisions / viable / unconv index sets, first viable state per test.
+Recorded: the x / u logs (NaN padded), conv / collisions / viable / unconv index sets, the initial states.  The scripted outcomes are
+not stored: ``scripted_inputs`` draws them again from their seeds, and ``input_digest`` (stored) pins them bit for bit.
 
     python tests/golden/make_ref_closed_loop.py   ->  tests/golden/ref_closed_loop.npz
 """
 import ast
+import hashlib
 import os
 import sys
 import types
@@ -47,6 +49,32 @@ def simulation_statements():
     return compile(ast.Module(body=tree.body[first:last + 1], type_ignores=[]), MPC, 'exec')
 
 
+def scripted_inputs(name, x_init):
+    """the scripted outcomes of the main and backup solves per (test, step) of one controller's run, drawn from its seed"""
+    rng = np.random.default_rng({'naive': 11, 'htwa': 12, 'receding': 13}[name])
+    status = rng.choice([0, 0, 0, 0, 4], size=(B, STEPS)).astype(np.int32)
+    status[:4, 5:16] = 4                                           # a long run of failures for the first tests -> abort
+    if name == 'receding':
+        status[4:6, :] = 0
+    xt = x_init[:, None, None, :] + 0.02 * rng.standard_normal((B, STEPS, N + 1, 10))
+    xt[:, :, :, 5:] *= rng.choice([0.05, 1.0, 4.0], size=(B, STEPS, 1, 1))
+    ut = 2.0 * rng.standard_normal((B, STEPS, N, 5))
+    bk_status = rng.choice([0, 0, 0, 4], size=(B, STEPS)).astype(np.int32)
+    bk_xt = x_init[:, None, None, :] + 0.02 * rng.standard_normal((B, STEPS, NB + 1, 10))
+    bk_xt[:, :, :, 5:] *= 0.1
+    bk_xt[1, :, -1, 5:] = 0.5                                      # test 1: the abort trajectory does not end at rest -> PD hold (mpc.py:143-144)
+    bk_ut = 0.5 * rng.standard_normal((B, STEPS, NB, 5))
+    return {'status': status, 'xt': xt, 'ut': ut, 'bk_status': bk_status, 'bk_xt': bk_xt, 'bk_ut': bk_ut}
+
+
+def input_digest(inputs):
+    """sha256 of the arrays of scripted_inputs, in key order"""
+    h = hashlib.sha256()
+    for k in sorted(inputs):
+        h.update(np.ascontiguousarray(inputs[k]).tobytes())
+    return h.hexdigest()
+
+
 class _Solver:
     def cost_set(self, *a): pass
     def set(self, *a): pass
@@ -61,26 +89,14 @@ def main():
     code = simulation_statements()
     out = {'N': N, 'NB': NB, 'B': B, 'STEPS': STEPS}
     for name, cls_name in CLASSES.items():
-        rng = np.random.default_rng({'naive': 11, 'htwa': 12, 'receding': 13}[name])
         prob, params, md = make_problem(name, N=N)
         orc = Oracle(prob, 1, 1)
         tol = params.tol_safe_set
         x_init = start_states(B, seed=17, vel=0.4)
         xg0 = np.repeat(x_init[:, None, :], N + 1, axis=1)
         ug0 = np.zeros((B, N, 5))
-        # ---- scripted solve outcomes per (test, step) ----
-        status = rng.choice([0, 0, 0, 0, 4], size=(B, STEPS)).astype(np.int32)
-        status[:4, 5:16] = 4                                           # a long run of failures for the first tests -> abort
-        if name == 'receding':
-            status[4:6, :] = 0
-        xt = x_init[:, None, None, :] + 0.02 * rng.standard_normal((B, STEPS, N + 1, 10))
-        xt[:, :, :, 5:] *= rng.choice([0.05, 1.0, 4.0], size=(B, STEPS, 1, 1))
-        ut = 2.0 * rng.standard_normal((B, STEPS, N, 5))
-        bk_status = rng.choice([0, 0, 0, 4], size=(B, STEPS)).astype(np.int32)
-        bk_xt = x_init[:, None, None, :] + 0.02 * rng.standard_normal((B, STEPS, NB + 1, 10))
-        bk_xt[:, :, :, 5:] *= 0.1
-        bk_xt[1, :, -1, 5:] = 0.5                                      # test 1: the abort trajectory does not end at rest -> PD hold (mpc.py:143-144)
-        bk_ut = 0.5 * rng.standard_normal((B, STEPS, NB, 5))
+        script = scripted_inputs(name, x_init)
+        status, xt, ut, bk_status, bk_xt, bk_ut = (script[k] for k in ('status', 'xt', 'ut', 'bk_status', 'bk_xt', 'bk_ut'))
 
         def state_in_bounds(x):
             return bool(np.all((x >= md.x_min - params.tol_x) & (x <= md.x_max + params.tol_x)))
@@ -153,8 +169,8 @@ def main():
         out[f'{name}_conv'] = np.array(sorted(ns['conv_idx']), dtype=np.int64); out[f'{name}_coll'] = np.array(sorted(set(ns['collisions_idx'])), dtype=np.int64)
         out[f'{name}_viable'] = np.array(sorted(ns['viable_idx']), dtype=np.int64); out[f'{name}_unconv'] = np.array(sorted(ns['unconv_idx']), dtype=np.int64)
         out[f'{name}_n_aborts'] = len(ns['x_viable'])
-        for k, v in (('status', status), ('xt', xt), ('ut', ut), ('bk_status', bk_status), ('bk_xt', bk_xt), ('bk_ut', bk_ut), ('x_init', x_init)):
-            out[f'{name}_{k}'] = v
+        out[f'{name}_x_init'] = x_init
+        out[f'{name}_input_digest'] = input_digest(script)
         print(name, 'conv', ns['conv_idx'], 'collisions', sorted(set(ns['collisions_idx'])), 'viable', sorted(ns['viable_idx']), 'unconv', ns['unconv_idx'],
               'aborts', len(ns['x_viable']))
     path = os.path.join(os.path.dirname(os.path.abspath(__file__)), 'ref_closed_loop.npz')

@@ -11,10 +11,13 @@ three things a step calls outside the class are stand-ins:
   * ``checkSafeConstraints``     the oracle's viability value >= -tol (the network is pinned separately);
   * ``model.integrate_naively``  the double integrator of env_model.py:63-71.
 What is recorded is everything the reference logic decides: control returned, abort flag, fails, receding index, viable state, next guess.
+The scripted inputs are not stored: ``scripted_inputs`` draws them again from their seed, given the few values they depend on (stored:
+the start states, the upper bound of joint 0, a colliding configuration per controller), and ``input_digest`` (stored) pins them bit for bit.
 
     python tests/golden/make_ref_controllers.py   ->  tests/golden/ref_controllers.npz
 """
 import ast
+import hashlib
 import os
 import sys
 import types
@@ -51,6 +54,47 @@ def reference_checks():
     return ns['RefChecks']()
 
 
+def scripted_inputs(x0, x_max0, colliding):
+    """the scripted guesses, states and solve outcomes of every controller, drawn in CLASSES order from one seeded stream:
+    {name: {xg0, ug0, x, status, xt, ut}}, the last four per step.  x0: start states [B, 10]; x_max0: upper bound of joint 0;
+    colliding[name]: a colliding configuration [10] or None."""
+    rng = np.random.default_rng(123)
+    out = {}
+    for name in CLASSES:
+        xg0 = np.repeat(x0[:, None, :], N + 1, axis=1) + 0.01 * rng.standard_normal((B, N + 1, 10))
+        ug0 = 0.5 * rng.standard_normal((B, N, 5))
+        rec = {k: [] for k in ('x', 'status', 'xt', 'ut')}
+        for step in range(STEPS):
+            x = x0 + 0.02 * step * rng.standard_normal((B, 10))
+            # scripted solve outcomes: mostly successes inside the bounds, some failures, some trajectories out of bounds / unsafe
+            status = rng.choice([0, 0, 0, 4, 2, 1], size=B).astype(np.int32)
+            if step in (3, 4, 5, 6, 7, 8, 9, 10):
+                status[:4] = 4                                          # a run of failures: exercises fails == N - 1 -> abort (N = 8)
+            xt = np.repeat(x[:, None, :], N + 1, axis=1) + 0.05 * rng.standard_normal((B, N + 1, 10))
+            xt[:, :, 5:] *= rng.choice([0.2, 1.0, 3.0], size=(B, 1, 1))   # slow / fast trajectories: safe / unsafe under the viability row
+            viol = rng.random(B) < 0.15
+            xt[viol, 3, 0] = x_max0 + 0.5                               # state-bound violation on a later row
+            if colliding[name] is not None:
+                late = rng.random(B) < 0.2
+                xt[late, 4, :5] = colliding[name][:5]                   # a collision on a LATER row: not seen by the reference's checkCollision
+                first = (rng.random(B) < 0.1) & ~late
+                xt[first, 0, :5] = colliding[name][:5]                  # a collision on row 0: seen
+            ut = rng.standard_normal((B, N, 5))
+            for k, v in zip(('x', 'status', 'xt', 'ut'), (x, status, xt, ut)):
+                rec[k].append(v)
+        out[name] = {'xg0': xg0, 'ug0': ug0, **{k: np.array(v) for k, v in rec.items()}}
+    return out
+
+
+def input_digest(inputs):
+    """sha256 of the arrays of scripted_inputs, controller by controller in CLASSES order, keys in sorted order"""
+    h = hashlib.sha256()
+    for name in CLASSES:
+        for k in sorted(inputs[name]):
+            h.update(np.ascontiguousarray(inputs[name][k]).tobytes())
+    return h.hexdigest()
+
+
 class _Solver:                                   # ocp_solver: the step methods only program flags / bounds on it
     def cost_set(self, *a): pass
     def set(self, *a): pass
@@ -62,11 +106,23 @@ def main():
     from oracle.oracle import Oracle
     ns = reference_classes()
     out = {'N': N, 'B': B, 'STEPS': STEPS}
-    rng = np.random.default_rng(123)
+    x0 = start_states(B, seed=7, vel=0.5)
+    colliding = {}
+    for name in CLASSES:
+        prob, params, md = make_problem(name, N=N)
+        cand = random_states(md, 4000, seed=3, vel_scale=0.0)
+        dd = Oracle(prob, 1, 1).kinematics(cand)[1]
+        bad = np.flatnonzero((dd < np.array(prob.pair_lo_chk)).any(axis=1) & ((cand >= md.x_min) & (cand <= md.x_max)).all(axis=1))
+        colliding[name] = cand[bad[0]] if len(bad) else None
+    x_max0 = float(md.x_max[0])
+    inputs = scripted_inputs(x0, x_max0, colliding)
+    out['x0'] = x0; out['x_max0'] = x_max0; out['input_digest'] = input_digest(inputs)
     for name, cls_name in CLASSES.items():
         prob, params, md = make_problem(name, N=N)
         orc = Oracle(prob, 1, 1)
         tol = params.tol_safe_set
+        assert float(md.x_max[0]) == x_max0
+        out[f'{name}_colliding'] = np.full(10, np.nan) if colliding[name] is None else colliding[name]
 
         # the reference's own predicates (env_model.py:170-177,236-243: checkStateConstraints -> bounds on every row and checkCollision,
         # which returns after the FIRST row of a trajectory), method bodies extracted unmodified; the capsule distance functions they
@@ -86,15 +142,9 @@ def main():
                                                                    abort_flag=bool(params.abort_flag), N=N, use_net=True),
                                       checkStateConstraints=check_state,
                                       integrate_naively=lambda x, u, dt=params.dt: np.hstack([x[:5] + dt * x[5:] + 0.5 * dt * dt * u, x[5:] + dt * u]))
-        cand = random_states(md, 4000, seed=3, vel_scale=0.0)
-        dd = orc.kinematics(cand)[1]
-        bad = np.flatnonzero((dd < np.array(prob.pair_lo_chk)).any(axis=1) & ((cand >= md.x_min) & (cand <= md.x_max)).all(axis=1))
-        colliding = cand[bad[0]] if len(bad) else None
-        rec = {k: [] for k in ('x', 'status', 'xt', 'ut', 'u', 'abort', 'fails', 'r', 'xv', 'xg', 'ug')}
+        rec = {k: [] for k in ('u', 'abort', 'fails', 'r', 'xv', 'xg', 'ug')}
         objs = []
-        x0 = start_states(B, seed=7, vel=0.5)
-        xg0 = np.repeat(x0[:, None, :], N + 1, axis=1) + 0.01 * rng.standard_normal((B, N + 1, 10))
-        ug0 = 0.5 * rng.standard_normal((B, N, 5))
+        xg0, ug0 = inputs[name]['xg0'], inputs[name]['ug0']
         for b in range(B):
             o = ns[cls_name].__new__(ns[cls_name])
             o.model = model; o.N = N; o.fails = 0; o.current_step = 0; o.r = N; o.abort_flag = model.params.abort_flag
@@ -102,23 +152,8 @@ def main():
             o.x_viable = np.copy(o.x_guess[-1]); o.ocp_solver = _Solver(); o.zl = np.zeros(0); o.zl_e = np.zeros(1)
             o.checkSafeConstraints = check_safe
             objs.append(o)
-        out[f'{name}_xg0'] = xg0; out[f'{name}_ug0'] = ug0
         for step in range(STEPS):
-            x = x0 + 0.02 * step * rng.standard_normal((B, 10))
-            # scripted solve outcomes: mostly successes inside the bounds, some failures, some trajectories out of bounds / unsafe
-            status = rng.choice([0, 0, 0, 4, 2, 1], size=B).astype(np.int32)
-            if step in (3, 4, 5, 6, 7, 8, 9, 10):
-                status[:4] = 4                                          # a run of failures: exercises fails == N - 1 -> abort (N = 8)
-            xt = np.repeat(x[:, None, :], N + 1, axis=1) + 0.05 * rng.standard_normal((B, N + 1, 10))
-            xt[:, :, 5:] *= rng.choice([0.2, 1.0, 3.0], size=(B, 1, 1))   # slow / fast trajectories: safe / unsafe under the viability row
-            viol = rng.random(B) < 0.15
-            xt[viol, 3, 0] = md.x_max[0] + 0.5                          # state-bound violation on a later row
-            if colliding is not None:
-                late = rng.random(B) < 0.2
-                xt[late, 4, :5] = colliding[:5]                         # a collision on a LATER row: not seen by the reference's checkCollision
-                first = (rng.random(B) < 0.1) & ~late
-                xt[first, 0, :5] = colliding[:5]                        # a collision on row 0: seen
-            ut = rng.standard_normal((B, N, 5))
+            x, status, xt, ut = (inputs[name][k][step] for k in ('x', 'status', 'xt', 'ut'))
             us, abs_, fl, rr, xv, xgn, ugn = [], [], [], [], [], [], []
             for b, o in enumerate(objs):
                 def solve(xx, o=o, b=b):
@@ -128,7 +163,7 @@ def main():
                 u, ab = o.step(x[b])
                 us.append(np.array(u, dtype=float)); abs_.append(bool(ab)); fl.append(o.fails); rr.append(getattr(o, 'r', N))
                 xv.append(np.array(o.x_viable, dtype=float)); xgn.append(o.x_guess.copy()); ugn.append(o.u_guess.copy())
-            for k, v in zip(('x', 'status', 'xt', 'ut', 'u', 'abort', 'fails', 'r', 'xv', 'xg', 'ug'), (x, status, xt, ut, us, abs_, fl, rr, xv, xgn, ugn)):
+            for k, v in zip(('u', 'abort', 'fails', 'r', 'xv', 'xg', 'ug'), (us, abs_, fl, rr, xv, xgn, ugn)):
                 rec[k].append(np.array(v))
         for k, v in rec.items():
             out[f'{name}_{k}'] = np.array(v)

@@ -3,6 +3,7 @@ where /root/reference is mounted): the one piece of the hot path that executes w
 They pin row a5 of SURVEY.md section 8 -- architecture, layer order, GELU(tanh), psi(x), c(x) and dc/dx -- on reference code instead of on
 a restatement: the oracle must reproduce the fp64 evaluation of the reference class to rounding, and the reference's fp32 evaluation
 (what its L4CasADi call computes) to fp32 accuracy; the CUDA kernels are held to the same vectors."""
+import functools
 import os
 
 import numpy as np
@@ -141,17 +142,28 @@ def test_capsule_distances_match_the_reference_function():
 CG = np.load(os.path.join(os.path.dirname(os.path.abspath(__file__)), 'golden', 'ref_controllers.npz'))
 
 
+@functools.lru_cache(maxsize=None)
+def controller_script():
+    """the scripted inputs the golden outputs were recorded with, drawn again from their seed (only the outputs are stored)"""
+    from tests.golden.make_ref_controllers import CLASSES, input_digest, scripted_inputs
+    colliding = {n: None if np.isnan(CG[f'{n}_colliding']).all() else CG[f'{n}_colliding'] for n in CLASSES}
+    script = scripted_inputs(CG['x0'], float(CG['x_max0']), colliding)
+    assert input_digest(script) == str(CG['input_digest']), 'the seeded stream no longer reproduces the recorded scripted inputs'
+    return script
+
+
 @pytest.mark.parametrize('name', ['naive', 'zerovel', 'st', 'stwa', 'htwa', 'receding', 'real_receding', 'constraint_everywhere'])
 def test_controller_state_machines_match_the_reference_classes(name):
     from oracle.oracle import Oracle
     from safe_mpc_b200 import abi
     N, B, steps = int(CG['N']), int(CG['B']), int(CG['STEPS'])
+    CI = controller_script()[name]
     prob, params, md = make_problem(name, N=N)
     orc = Oracle(prob, B, 1)
-    orc.set_guess(CG[f'{name}_xg0'], CG[f'{name}_ug0'])
+    orc.set_guess(CI['xg0'], CI['ug0'])
     orc.reset_controller()
     for s in range(steps):
-        u, ab = orc.controller_step_scripted(CG[f'{name}_x'][s], CG[f'{name}_status'][s], CG[f'{name}_xt'][s], CG[f'{name}_ut'][s])
+        u, ab = orc.controller_step_scripted(CI['x'][s], CI['status'][s], CI['xt'][s], CI['ut'][s])
         where = f'{name}, step {s}'
         np.testing.assert_array_equal(ab, CG[f'{name}_abort'][s], err_msg=f'abort flag, {where}')
         np.testing.assert_array_equal(orc.get_state(abi.STATE_FAILS), CG[f'{name}_fails'][s], err_msg=f'fails, {where}')
@@ -178,17 +190,19 @@ def test_closed_loop_matches_the_reference_script(name):
     from oracle.oracle import Oracle, OracleSim
     from safe_mpc_b200 import abi
     N, NB, B, steps = int(LG['N']), int(LG['NB']), int(LG['B']), int(LG['STEPS'])
+    from tests.golden.make_ref_closed_loop import input_digest, scripted_inputs
     prob, params, md = make_problem(name, N=N)
     bprob, _, _ = make_problem('backup', cost='zero', N=NB)
     main, bk = Oracle(prob, B, 1), Oracle(bprob, B, 1)
     x_init = LG[f'{name}_x_init']
+    SI = scripted_inputs(name, x_init)                    # drawn again from its seed: only the outputs are stored
+    assert input_digest(SI) == str(LG[f'{name}_input_digest']), 'the seeded stream no longer reproduces the recorded scripted inputs'
     main.set_guess(np.repeat(x_init[:, None, :], N + 1, axis=1).copy(), np.zeros((B, N, abi.NU)))
     main.reset_controller()
     sim = OracleSim(main, bk, steps)
     sim.reset(x_init)
     for j in range(steps):
-        sim.set_script(LG[f'{name}_status'][:, j], LG[f'{name}_xt'][:, j], LG[f'{name}_ut'][:, j],
-                       LG[f'{name}_bk_status'][:, j], LG[f'{name}_bk_xt'][:, j], LG[f'{name}_bk_ut'][:, j])
+        sim.set_script(SI['status'][:, j], SI['xt'][:, j], SI['ut'][:, j], SI['bk_status'][:, j], SI['bk_xt'][:, j], SI['bk_ut'][:, j])
         sim.step()
     x, u = sim.log()
     gx, gu = LG[f'{name}_x'], LG[f'{name}_u']
