@@ -472,6 +472,115 @@ __global__ void __launch_bounds__(32 * SP_WARPS, QS_SP_MINB) qs_step_kernel(cons
   qs_step(*dP, q, w / (q.N + 1), threadIdx.x & 31, w % (q.N + 1), kk, MODE);
 }
 
+// ---------------------------------------------------------------------------------------------------------------
+// step, staged form: the same warp per (tile, stage) and lane per problem, and the same qs_step instruction stream per lane, with
+// its operands read from a per-warp ring of SR_SLOTS chunks in shared memory instead of global memory (qp_split.cuh: QsStepGlobal,
+// qs_sp).  The lowest active lane fills the ring with cp.async.bulk copies (mbarrier completion), SR_SLOTS - 1 chunks ahead of the
+// arithmetic, so the loads of the next phases are in flight while a phase computes: the thread form waits for the loads of each of its
+// ten phases in turn (ncu, round 2: 16 of 20 stall cycles per issue on long_scoreboard).  Slot layout = global layout, [field][lane].
+// The inputs (st, st2, prod, the record, the iterate) were written by earlier kernels and nothing this kernel stores is fetched by it
+// again, so no proxy fence is needed; the stores go to global memory as in the thread form.
+// ---------------------------------------------------------------------------------------------------------------
+constexpr int SR_SLOTS = 3;
+constexpr int SR_SLOT_BYTES = qs_chunk_max_bytes();                  // 9 KB (fp64) / 7 KB (fp32 storage)
+constexpr size_t SR_WARP_BYTES = ((size_t)SR_SLOTS * SR_SLOT_BYTES + 8 * SR_SLOTS + 127) / 128 * 128;   // (bulk copies: 16-byte aligned slots)
+constexpr size_t SR_SMEM = SP_WARPS * SR_WARP_BYTES;
+static_assert(SR_SLOT_BYTES % 128 == 0 && SR_WARP_BYTES % 128 == 0, "bulk-copy alignment");
+static_assert(QS_SP_MINB * (SR_SMEM + 1024) <= 228 * 1024, "the ring keeps QS_SP_MINB CTAs per SM resident");
+
+template <int MODE>
+struct StepRing {
+  unsigned char* sm;       // SR_SLOTS slots, then SR_SLOTS mbarriers
+  QsBufs q;                // (kernel parameters: read from the constant bank when a copy is issued)
+  size_t blk;              // tile (N + 1) + k
+  const double* itp;       // iterate q.it[kk & 1]
+  StageFlags F;
+  unsigned mask;           // lanes that run qs_step
+  int ln;
+  bool lead;               // lowest lane of the mask: issues the copies
+  __device__ __forceinline__ uint64_t* bar(int s) const { return reinterpret_cast<uint64_t*>(sm + (size_t)SR_SLOTS * SR_SLOT_BYTES) + s; }
+  __device__ __forceinline__ const void* gsrc(const QsPiece& p) const {
+    switch (p.a) {
+      case QA_IT: return itp + (blk * NIT + p.f0) * TL;
+      case QA_ST: return q.st + (blk * NIT + p.f0) * TL;
+      case QA_ST2: return q.st2 + (blk * NS2 + p.f0) * TL;
+      case QA_REC: return q.rec + (blk * REC + p.f0) * TL;
+      default: return q.prod + (blk * NPROD + p.f0) * TL;
+    }
+  }
+  __device__ __forceinline__ void issue(int c) {
+    if (!lead || c >= QSC_N) return;
+    const bool on = qs_chunk_on(c, F);
+    const uint32_t b = smem_u32(bar(c % SR_SLOTS));
+    asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(b), "r"(on ? (uint32_t)qs_chunk_bytes(MODE, c) : 0u) : "memory");
+    if (!on) return;
+    uint32_t dst = smem_u32(sm + (size_t)(c % SR_SLOTS) * SR_SLOT_BYTES);
+#pragma unroll
+    for (int i = 0; i < QSC_PIECES; ++i) {
+      const QsPiece p = qs_sp(MODE, c, i);
+      if (p.n == 0) continue;
+      asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];" ::"r"(dst), "l"(gsrc(p)),
+                   "r"((uint32_t)qs_sp_bytes(p)), "r"(b) : "memory");
+      dst += qs_sp_bytes(p);
+    }
+  }
+  __device__ __forceinline__ void start() {
+    if (lead) {
+#pragma unroll
+      for (int s = 0; s < SR_SLOTS; ++s) asm volatile("mbarrier.init.shared::cta.b64 [%0], 1;" ::"r"(smem_u32(bar(s))));
+      asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
+#pragma unroll
+      for (int c = 0; c < SR_SLOTS; ++c) issue(c);
+    }
+    __syncwarp(mask);
+  }
+  __device__ __forceinline__ void acquire(int c) const {
+    const uint32_t addr = smem_u32(bar(c % SR_SLOTS)), par = (uint32_t)((c / SR_SLOTS) & 1);
+    uint32_t ok;
+    do {
+      asm volatile("{ .reg .pred p; mbarrier.try_wait.parity.shared::cta.b64 p, [%1], %2; selp.u32 %0, 1, 0, p; }" : "=r"(ok) : "r"(addr), "r"(par) : "memory");
+    } while (!ok);
+  }
+  // every lane has read chunk c: its slot takes chunk c + SR_SLOTS
+  __device__ __forceinline__ void release(int c) {
+    __syncwarp(mask);
+    issue(c + SR_SLOTS);
+  }
+  template <class T>
+  __device__ __forceinline__ double ld(int c, int a, int f) const {
+    return (double)*reinterpret_cast<const T*>(sm + (size_t)(c % SR_SLOTS) * SR_SLOT_BYTES + qs_chunk_off(MODE, c, a, f) + ln * sizeof(T));
+  }
+  __device__ __forceinline__ double it(int c, int f) const { return ld<double>(c, QA_IT, f); }
+  __device__ __forceinline__ double st(int c, int f) const { return ld<qs_real>(c, QA_ST, f); }
+  __device__ __forceinline__ double st2(int c, int f) const { return ld<qs_real>(c, QA_ST2, f); }
+  __device__ __forceinline__ double prod(int c, int f) const { return ld<qs_real>(c, QA_PROD, f); }
+  __device__ __forceinline__ double rec(int c, int f) const { return ld<qs_real>(c, QA_REC, f); }
+};
+
+template <int MODE>
+__global__ void __launch_bounds__(32 * SP_WARPS, QS_SP_MINB) qs_step_ring_kernel(const smpc_problem_t* __restrict__ dP, QsBufs q, int T, int kk) {
+  extern __shared__ __align__(128) unsigned char sr_sm[];
+  const int wi = threadIdx.x >> 5, lane = threadIdx.x & 31;
+  const int w = blockIdx.x * SP_WARPS + wi;
+  if (w >= T * (q.N + 1)) return;
+  const int N = q.N, tile = w / (N + 1), k = w % (N + 1);
+  const int32_t* pi = q.pi + qs_pb(tile, NPI, lane);
+  const bool on = QF(pi, J_ACT) && (MODE != 2 || QF(pi, J_REDO));   // the lanes qs_step does not return from at once
+  const unsigned mask = __ballot_sync(0xffffffffu, on);
+  if (!on) return;
+  StepRing<MODE> r;
+  r.sm = sr_sm + (size_t)wi * SR_WARP_BYTES;
+  r.q = q;
+  r.blk = (size_t)tile * (N + 1) + k;
+  r.itp = q.it[kk & 1];
+  r.F = qs_flags(*dP, k);
+  r.mask = mask;
+  r.ln = lane;
+  r.lead = lane == __ffs(mask) - 1;
+  r.start();
+  qs_step(*dP, q, tile, lane, k, kk, MODE, r);
+}
+
 __global__ void __launch_bounds__(32) qs_ctl_kernel(const smpc_problem_t* __restrict__ dP, QsBufs q, int kk, int32_t* status, int32_t* qp_iter,
                                                      int32_t* qp_status, double* qp_res, int* counters) {
   const bool on = qs_ctl<16>(*dP, q, blockIdx.x, threadIdx.x, kk, status, qp_iter, qp_status, qp_res);
@@ -1123,6 +1232,7 @@ struct QpSolver {
   int tail_which = 3;           // development: bit 0 / 1 = the factorising / the vector sweep may use the warp-per-problem form (SMPC_QP_TAIL_WHICH)
   bool split_ric1 = true;       // two warps per tile in the factorising Riccati sweep (SMPC_QP_RIC1=single selects the one-warp form)
   bool coop_prep = true;        // kk >= 1: four-warp cooperative prep with TMA-staged inputs (SMPC_QP_PREP=thread selects the thread-per-stage form)
+  bool ring_step = true;        // step kernels read their operands from a per-warp ring of bulk copies (SMPC_QP_STEP=thread: straight from global memory)
   bool profile = false;         // record one event pair per kernel of the next solves (smpc_set_profiling)
   double prof_ms[SMPC_PROF_N] = {0};
   int32_t prof_n[SMPC_PROF_N] = {0};
@@ -1171,6 +1281,10 @@ QpSolver* qp_create(int B, int N, int iter_max, bool keep_slots, cudaStream_t st
   if (e == cudaSuccess) e = cudaFuncSetAttribute(qs_prep_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)PREP_SMEM);
   if (e == cudaSuccess) e = cudaFuncSetAttribute(qs_prep_coop_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)PC_SMEM);
   if (const char* pe = getenv("SMPC_QP_PREP")) s->coop_prep = strcmp(pe, "thread") != 0;
+  if (e == cudaSuccess) e = cudaFuncSetAttribute(qs_step_ring_kernel<0>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)SR_SMEM);
+  if (e == cudaSuccess) e = cudaFuncSetAttribute(qs_step_ring_kernel<1>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)SR_SMEM);
+  if (e == cudaSuccess) e = cudaFuncSetAttribute(qs_step_ring_kernel<2>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)SR_SMEM);
+  if (const char* se = getenv("SMPC_QP_STEP")) s->ring_step = strcmp(se, "thread") != 0;
   if (e == cudaSuccess) e = cudaFuncSetAttribute(qs_ric1_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)RIC1_SMEM);
   if (e == cudaSuccess) e = cudaFuncSetAttribute(qs_ric1x_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)RIC1X_SMEM);
   if (const char* re = getenv("SMPC_QP_RIC1")) s->split_ric1 = strcmp(re, "single") != 0;
@@ -1361,9 +1475,14 @@ struct DeviceBackend {
     }
     count();
   }
+  template <int MODE>
+  void step_pass(cudaStream_t stm_, int kk, bool ring) {
+    if (ring) qs_step_ring_kernel<MODE><<<sp_grid(), 32 * SP_WARPS, SR_SMEM, stm_>>>(dP, g->q, tl(), kk);
+    else qs_step_kernel<MODE><<<sp_grid(), 32 * SP_WARPS, 0, stm_>>>(dP, g->q, tl(), kk);
+  }
   void step(int kk, int mode) {
-    if (mode == 0) { cudaStream_t stm_ = st(false); tr0("qs_step_kernel<0>", stm_); qs_step_kernel<0><<<sp_grid(), 32 * SP_WARPS, 0, stm_>>>(dP, g->q, tl(), kk); tr1(stm_); }
-    else if (mode == 1) { cudaStream_t stm_ = st(false); tr0("qs_step_kernel<1>", stm_); qs_step_kernel<1><<<sp_grid(), 32 * SP_WARPS, 0, stm_>>>(dP, g->q, tl(), kk); tr1(stm_); }
+    if (mode == 0) { cudaStream_t stm_ = st(false); tr0("qs_step_kernel<0>", stm_); step_pass<0>(stm_, kk, s->ring_step); tr1(stm_); }
+    else if (mode == 1) { cudaStream_t stm_ = st(false); tr0("qs_step_kernel<1>", stm_); step_pass<1>(stm_, kk, s->ring_step); tr1(stm_); }
     else {
       cudaStream_t stm_ = st(false);
       tr0("qs_step_kernel<2>", stm_);
@@ -1372,7 +1491,7 @@ struct DeviceBackend {
       if (n_redo_kk == kk && n_redo_last > 0 && n_redo_last <= lim) {
         qs_redo_list_kernel<<<n_redo_last, RL_THREADS, 0, stm_>>>(dP, g->q, kk, g->redo_list, g->counters + 2 * kk + 1);
         red_done = true;
-      } else qs_step_kernel<2><<<sp_grid(), 32 * SP_WARPS, 0, stm_>>>(dP, g->q, tl(), kk);
+      } else step_pass<2>(stm_, kk, s->ring_step);
       tr1(stm_);
     }
     count();

@@ -133,15 +133,18 @@ SMPC_HD StageFlags qs_flags(const smpc_problem_t& P, int k) {
 }
 
 // box of dx_j at stage k (controller.py:49-55,144-145,300-306,530-536,701-707)
-SMPC_HD void qs_box(const smpc_problem_t& P, const QsBufs& q, int tile, int lane, int k, int j, double x0j, int rrec, double& lo, double& hi) {
+// xk: x_j of the guess at stage k (record field SMPC_REC_X + j)
+SMPC_HD void qs_box_x(const smpc_problem_t& P, const QsBufs& q, int tile, int lane, int k, int j, double xk, double x0j, int rrec, double& lo, double& hi) {
   const int N = q.N;
-  const double xk = QF(q.rec + qs_blk(tile, N, k, REC, lane), SMPC_REC_X + j);
   if (k == 0) { lo = x0j - xk; hi = lo; }
   else if (k == N) { lo = P.lbx_e[j] - xk; hi = P.ubx_e[j] - xk; }
   else if (P.controller == SMPC_CTRL_REAL_RECEDING) {
     if (k == rrec) { const double c = QF(q.rec + qs_blk(tile, N, k + 1, REC, lane), SMPC_REC_X + j); lo = c - 1e-3 - xk; hi = c + 1e-3 - xk; }
     else { lo = P.x_min[j] - xk; hi = P.x_max[j] - xk; }
   } else { lo = P.lbx[j] - xk; hi = P.ubx[j] - xk; }
+}
+SMPC_HD void qs_box(const smpc_problem_t& P, const QsBufs& q, int tile, int lane, int k, int j, double x0j, int rrec, double& lo, double& hi) {
+  qs_box_x(P, q, tile, lane, k, j, QF(q.rec + qs_blk(tile, q.N, k, REC, lane), SMPC_REC_X + j), x0j, rrec, lo, hi);
 }
 // cold start of a box row: primal moved inside, slacks >= thr0
 SMPC_HD double qs_zinit(double lo, double hi, double& tl, double& tu) {
@@ -1074,8 +1077,100 @@ SMPC_HD void qs_ric2(const smpc_problem_t& P, const QsBufs& q, int tile, W& w) {
 // step: recover (dlam, dt, dslack) of every row from dz, step-length partials.   thread = (problem, stage)
 //   mode 0 (affine): stores dlam*dt per slot and the corrector gradient terms v1, v2
 //   mode 1 / 2 (corrector / centering): stores the step
+//
+// Operand source.  qs_step reads its stage block (iterate, step or centering direction, products, record) through a policy S:
+//   S.it(c, f), S.st(c, f), S.st2(c, f), S.prod(c, f), S.rec(c, f)   field f of that block, widened to fp64
+//   S.acquire(c) / S.release(c)                                       chunk c is about to be read / has been read for the last time
+// The chunks c = 0 .. QSC_N - 1 follow the load phases in the order they run (table qs_sp below).  QsStepGlobal reads global memory
+// (acquire / release are no-ops); the staged kernels of qp.cu read a per-warp ring of chunks that bulk copies fill ahead of the
+// arithmetic.  Every lane runs the same instructions on the same values in both: a problem's result does not depend on the source.
+// Stores go to global memory in both.
 // ================================================================================================================
-SMPC_HD void qs_step(const smpc_problem_t& P, const QsBufs& q, int tile, int lane, int k, int kk, int mode) {
+enum { QA_NONE = 0, QA_IT, QA_ST, QA_ST2, QA_REC, QA_PROD };
+struct QsPiece { int a, f0, n; };   // fields [f0, f0 + n) of one array of the stage block
+enum { QSC_N = 16, QSC_PIECES = 7 };
+// both sides of the row slots [s0, s0 + n): lam (lower, upper), t (lower, upper), and in mode 1 the products
+SMPC_HD constexpr QsPiece qs_sp_rows(int mode, int s0, int n, int i) {
+  return i < 4 ? QsPiece{QA_IT, ((i & 2) ? I_T : I_LAM) + (i & 1) * QNR + s0, n}
+               : (mode == 1 && i < 6) ? QsPiece{QA_PROD, (i & 1) * QNR + s0, n} : QsPiece{QA_NONE, 0, 0};
+}
+// piece i of chunk c in `mode` (n = 0: past the last piece).  The record ranges are cut so that no chunk exceeds 36 fields: the torque
+// rows in pieces of two rows, each with the five torque values the rows are compared against; the Jacobians are fetched again for the
+// corrector terms of mode 0 (they were read three phases earlier, from L2 by then).
+SMPC_HD constexpr QsPiece qs_sp(int mode, int c, int i) {
+  constexpr QsPiece no{QA_NONE, 0, 0};
+  switch (c) {
+    case 0: return i == 0 ? QsPiece{QA_IT, I_Z, 15} : i == 1 ? QsPiece{mode == 2 ? QA_ST2 : QA_ST, I_Z, 15} : no;   // z, dz
+    case 1: return i == 0 ? QsPiece{QA_REC, SMPC_REC_X, 5} : qs_sp_rows(mode, 0, 5, i - 1);                     // box rows 0-4
+    case 2: return i == 0 ? QsPiece{QA_REC, SMPC_REC_X + 5, 5} : qs_sp_rows(mode, 5, 5, i - 1);                 // box rows 5-9
+    case 3: return i == 0 ? QsPiece{QA_REC, SMPC_REC_TAU, 35} : no;                                             // tau, rows 0-1 of d tau
+    case 4: return i == 0 ? QsPiece{QA_REC, SMPC_REC_TAU, 5} : i == 1 ? QsPiece{QA_REC, SMPC_REC_JTAU + 30, 30} : no;
+    case 5: return i == 0 ? QsPiece{QA_REC, SMPC_REC_TAU, 5} : i == 1 ? QsPiece{QA_REC, SMPC_REC_JTAU + 60, 15} : no;
+    case 6: return i == 0 ? QsPiece{QA_REC, SMPC_REC_DIST, 36} : no;                                            // capsule rows
+    case 7: return i == 0 ? QsPiece{QA_REC, SMPC_REC_NN, 11} : no;                                              // viability row
+    case 8: return qs_sp_rows(mode, 10, 5, i);                                                                  // torque slots
+    case 9: return mode == 0 && i == 0 ? QsPiece{QA_REC, SMPC_REC_JTAU, 30} : no;
+    case 10: return mode == 0 && i == 0 ? QsPiece{QA_REC, SMPC_REC_JTAU + 30, 30} : no;
+    case 11: return mode == 0 && i == 0 ? QsPiece{QA_REC, SMPC_REC_JTAU + 60, 15} : no;
+    case 12: return qs_sp_rows(mode, 15, 6, i);                                                                 // capsule slots
+    case 13: return mode == 0 && i == 0 ? QsPiece{QA_REC, SMPC_REC_JDIST, 30} : no;
+    case 14:                                                                                                    // viability slots, slacks
+      return i == 0 ? QsPiece{QA_REC, SMPC_REC_NN, 11} : i == 1 ? QsPiece{QA_IT, I_LAM + 21, 1} : i == 2 ? QsPiece{QA_IT, I_LAM + QNR + 21, 1}
+           : i == 3 ? QsPiece{QA_IT, I_T + 21, 1} : i == 4 ? QsPiece{QA_IT, I_T + QNR + 21, 8}   // t (upper) + the six slack fields
+           : mode == 1 && i == 5 ? QsPiece{QA_PROD, 21, 1} : mode == 1 && i == 6 ? QsPiece{QA_PROD, QNR + 21, 3} : no;
+    case 15: return mode == 2 && i == 0 ? QsPiece{QA_ST2, I_PIM, 10} : no;                                     // dpi of the centering direction
+    default: return no;
+  }
+}
+static_assert(I_T + QNR + 21 + 8 <= NIT && I_SLK + 6 <= I_T + QNR + 21 + 8, "viability chunk covers the slacks");
+SMPC_HD constexpr int qs_sp_esz(int a) { return a == QA_IT ? (int)sizeof(double) : (int)sizeof(qs_real); }
+SMPC_HD constexpr int qs_sp_bytes(const QsPiece& p) { return p.n * TL * qs_sp_esz(p.a); }
+SMPC_HD constexpr int qs_chunk_bytes(int mode, int c) {
+  int b = 0;
+  for (int i = 0; i < QSC_PIECES; ++i) b += qs_sp_bytes(qs_sp(mode, c, i));
+  return b;
+}
+SMPC_HD constexpr int qs_chunk_max_bytes() {
+  int m = 0;
+  for (int mode = 0; mode < 3; ++mode)
+    for (int c = 0; c < QSC_N; ++c) m = qs_chunk_bytes(mode, c) > m ? qs_chunk_bytes(mode, c) : m;
+  return m;
+}
+// byte offset of field f of array a inside chunk c (layout [field][lane], pieces in table order); -1: not in the chunk
+SMPC_HD constexpr int qs_chunk_off(int mode, int c, int a, int f) {
+  int off = 0;
+  for (int i = 0; i < QSC_PIECES; ++i) {
+    const QsPiece p = qs_sp(mode, c, i);
+    if (p.a == a && f >= p.f0 && f < p.f0 + p.n) return off + (f - p.f0) * TL * qs_sp_esz(a);
+    off += qs_sp_bytes(p);
+  }
+  return -1;
+}
+// chunks the stage does not use (its rows are absent) are skipped: nothing is fetched
+SMPC_HD bool qs_chunk_on(int c, const StageFlags& F) {
+  return (c >= 3 && c <= 5) || (c >= 8 && c <= 11) ? F.tau : (c == 6 || c == 12 || c == 13) ? F.dist : (c == 7 || c == 14) ? F.nn : true;
+}
+
+struct QsStepGlobal {
+  const qs_real* rec_;
+  const double* it_;
+  const qs_real* st_;
+  const qs_real* st2_;
+  const qs_real* prod_;
+  SMPC_HD QsStepGlobal(const QsBufs& q, int tile, int lane, int k, int kk)
+      : rec_(q.rec + qs_blk(tile, q.N, k, REC, lane)), it_(q.it[kk & 1] + qs_blk(tile, q.N, k, NIT, lane)), st_(q.st + qs_blk(tile, q.N, k, NIT, lane)),
+        st2_(q.st2 + qs_blk(tile, q.N, k, NS2, lane)), prod_(q.prod + qs_blk(tile, q.N, k, NPROD, lane)) {}
+  SMPC_HD void acquire(int) const {}
+  SMPC_HD void release(int) const {}
+  SMPC_HD double it(int, int f) const { return QF(it_, f); }
+  SMPC_HD double st(int, int f) const { return QF(st_, f); }
+  SMPC_HD double st2(int, int f) const { return QF(st2_, f); }
+  SMPC_HD double prod(int, int f) const { return QF(prod_, f); }
+  SMPC_HD double rec(int, int f) const { return QF(rec_, f); }
+};
+
+template <class S>
+SMPC_HD void qs_step(const smpc_problem_t& P, const QsBufs& q, int tile, int lane, int k, int kk, int mode, S& src) {
   const int N = q.N;
   const int32_t* pi = q.pi + qs_pb(tile, NPI, lane);
   if (!QF(pi, J_ACT)) return;
@@ -1083,21 +1178,20 @@ SMPC_HD void qs_step(const smpc_problem_t& P, const QsBufs& q, int tile, int lan
   const double* pd = q.pd + qs_pb(tile, NPD, lane);
   const int rrec = QF(pi, J_R);
   const double sigmu = mode == 0 ? 0.0 : QF(pd, D_SIGMU);
-  const qs_real* rec = q.rec + qs_blk(tile, N, k, REC, lane);
-  const double* it = q.it[kk & 1] + qs_blk(tile, N, k, NIT, lane);
   qs_real* st = q.st + qs_blk(tile, N, k, NIT, lane);
   qs_real* prod = q.prod + qs_blk(tile, N, k, NPROD, lane);
   const StageFlags F = qs_flags(P, k);
   double z[15], dz[15];
+  src.acquire(0);
   if (mode == 2) {
     // the centering direction was computed by ric2 next to the corrector: it becomes the step of this problem
-    const qs_real* st2 = q.st2 + qs_blk(tile, N, k, NS2, lane);
 #pragma unroll
-    for (int i = 0; i < 15; ++i) { z[i] = QF(it, I_Z + i); dz[i] = QF(st2, I_Z + i); }
+    for (int i = 0; i < 15; ++i) { z[i] = src.it(0, I_Z + i); dz[i] = src.st2(0, I_Z + i); }
   } else {
 #pragma unroll
-    for (int i = 0; i < 15; ++i) { z[i] = QF(it, I_Z + i); dz[i] = QF(st, I_Z + i); }
+    for (int i = 0; i < 15; ++i) { z[i] = src.it(0, I_Z + i); dz[i] = src.st(0, I_Z + i); }
   }
+  src.release(0);
   // step length = min over the slots of lam / (-dlam), t / (-dt) (negative steps only), kept as a fraction an / ad and
   // compared by cross-multiplication: one division per thread instead of two per slot
   double an = 1.0, ad = 1.0, s_lin = 0.0, s_quad = 0.0;
@@ -1124,13 +1218,17 @@ SMPC_HD void qs_step(const smpc_problem_t& P, const QsBufs& q, int tile, int lan
     double lo[10], hi[10], bl[20], bt[20], bp[20];
 #pragma unroll
     for (int j = 0; j < 10; ++j) {
-      qs_box(P, q, tile, lane, k, j, QF(pd, D_X0 + j), rrec, lo[j], hi[j]);
+      const int c = j < 5 ? 1 : 2;
+      if (j == 0) src.acquire(1);
+      if (j == 5) { src.release(1); src.acquire(2); }
+      qs_box_x(P, q, tile, lane, k, j, src.rec(c, SMPC_REC_X + j), QF(pd, D_X0 + j), rrec, lo[j], hi[j]);
 #pragma unroll
       for (int h = 0; h < 2; ++h) {
-        bl[h * 10 + j] = QF(it, I_LAM + h * QNR + j); bt[h * 10 + j] = QF(it, I_T + h * QNR + j);
-        bp[h * 10 + j] = mode == 1 ? QF(prod, h * QNR + j) : 0.0;
+        bl[h * 10 + j] = src.it(c, I_LAM + h * QNR + j); bt[h * 10 + j] = src.it(c, I_T + h * QNR + j);
+        bp[h * 10 + j] = mode == 1 ? src.prod(c, h * QNR + j) : 0.0;
       }
     }
+    src.release(2);
 #pragma unroll
     for (int j = 0; j < 10; ++j) {
       double e1 = 0.0, e2 = 0.0;
@@ -1146,50 +1244,69 @@ SMPC_HD void qs_step(const smpc_problem_t& P, const QsBufs& q, int tile, int lan
   if (F.tau) {
 #pragma unroll
     for (int r = 0; r < 5; ++r) {
+      const int cj = 3 + r / 2;        // chunk of d tau row r (with tau)
+      if (r == 0) src.acquire(3);
+      if (r == 2 || r == 4) { src.release(cj - 1); src.acquire(cj); }
       double az = 0.0, adz = 0.0;
 #pragma unroll
-      for (int c = 0; c < 15; ++c) { const double jv = QF(rec, SMPC_REC_JTAU + r * 15 + c); az += jv * z[c]; adz += jv * dz[c]; }
-      const double v = QF(rec, SMPC_REC_TAU + r);
+      for (int c = 0; c < 15; ++c) { const double jv = src.rec(cj, SMPC_REC_JTAU + r * 15 + c); az += jv * z[c]; adz += jv * dz[c]; }
+      const double v = src.rec(cj, SMPC_REC_TAU + r);
       azg[r] = az; adg[r] = adz; glo[r] = P.tau_min[r] - v; ghi[r] = P.tau_max[r] - v;
     }
+    src.release(5);
+  } else {
+    for (int c = 3; c <= 5; ++c) { src.acquire(c); src.release(c); }
   }
+  src.acquire(6);
   if (F.dist) {
 #pragma unroll
     for (int p = 0; p < 6; ++p) {
       double az = 0.0, adz = 0.0;
 #pragma unroll
-      for (int c = 0; c < 5; ++c) { const double jv = QF(rec, SMPC_REC_JDIST + p * 5 + c); az += jv * z[5 + c]; adz += jv * dz[5 + c]; }
-      const double v = QF(rec, SMPC_REC_DIST + p);
+      for (int c = 0; c < 5; ++c) { const double jv = src.rec(6, SMPC_REC_JDIST + p * 5 + c); az += jv * z[5 + c]; adz += jv * dz[5 + c]; }
+      const double v = src.rec(6, SMPC_REC_DIST + p);
       azg[5 + p] = az; adg[5 + p] = adz; glo[5 + p] = P.pair_lo_ocp[p] - v; ghi[5 + p] = P.pair_hi - v;
     }
   }
+  src.release(6);
+  src.acquire(7);
   if (F.nn) {
     double az = 0.0, adz = 0.0;
 #pragma unroll
-    for (int c = 0; c < 10; ++c) { const double jv = QF(rec, SMPC_REC_JNN + c); az += jv * z[5 + c]; adz += jv * dz[5 + c]; }
-    const double v = QF(rec, SMPC_REC_NN);
+    for (int c = 0; c < 10; ++c) { const double jv = src.rec(7, SMPC_REC_JNN + c); az += jv * z[5 + c]; adz += jv * dz[5 + c]; }
+    const double v = src.rec(7, SMPC_REC_NN);
     azg[11] = az; adg[11] = adz; glo[11] = 0.0 - v; ghi[11] = 1e6 - v;
   }
+  src.release(7);
   if (F.tau) {
     double gl[10], gt[10], gp[10];
+    src.acquire(8);
 #pragma unroll
     for (int r = 0; r < 5; ++r)
 #pragma unroll
       for (int h = 0; h < 2; ++h) {
         const int slot = h * QNR + 10 + r;
-        gl[h * 5 + r] = QF(it, I_LAM + slot); gt[h * 5 + r] = QF(it, I_T + slot); gp[h * 5 + r] = mode == 1 ? QF(prod, slot) : 0.0;
+        gl[h * 5 + r] = src.it(8, I_LAM + slot); gt[h * 5 + r] = src.it(8, I_T + slot); gp[h * 5 + r] = mode == 1 ? src.prod(8, slot) : 0.0;
       }
+    src.release(8);
 #pragma unroll
     for (int r = 0; r < 5; ++r) {
+      const int cj = 9 + r / 2;        // chunk of d tau row r (corrector terms, mode 0)
+      if (r == 0) src.acquire(9);
+      if (r == 2 || r == 4) { src.release(cj - 1); src.acquire(cj); }
       double e1 = 0.0, e2 = 0.0;
       side(10 + r, 1.0, azg[r], adg[r], glo[r], gl[r], gt[r], gp[r], e1, e2);
       side(QNR + 10 + r, -1.0, azg[r], adg[r], ghi[r], gl[5 + r], gt[5 + r], gp[5 + r], e1, e2);
       if (mode == 0) {
 #pragma unroll
-        for (int c = 0; c < 15; ++c) { const double jv = QF(rec, SMPC_REC_JTAU + r * 15 + c); v1[c] += jv * e1; v2[c] += jv * e2; }
+        for (int c = 0; c < 15; ++c) { const double jv = src.rec(cj, SMPC_REC_JTAU + r * 15 + c); v1[c] += jv * e1; v2[c] += jv * e2; }
       }
     }
+    src.release(11);
+  } else {
+    for (int c = 8; c <= 11; ++c) { src.acquire(c); src.release(c); }
   }
+  src.acquire(12);
   if (F.dist) {
     double gl[12], gt[12], gp[12];
 #pragma unroll
@@ -1197,8 +1314,10 @@ SMPC_HD void qs_step(const smpc_problem_t& P, const QsBufs& q, int tile, int lan
 #pragma unroll
       for (int h = 0; h < 2; ++h) {
         const int slot = h * QNR + 15 + p;
-        gl[h * 6 + p] = QF(it, I_LAM + slot); gt[h * 6 + p] = QF(it, I_T + slot); gp[h * 6 + p] = mode == 1 ? QF(prod, slot) : 0.0;
+        gl[h * 6 + p] = src.it(12, I_LAM + slot); gt[h * 6 + p] = src.it(12, I_T + slot); gp[h * 6 + p] = mode == 1 ? src.prod(12, slot) : 0.0;
       }
+    src.release(12);
+    src.acquire(13);
 #pragma unroll
     for (int p = 0; p < 6; ++p) {
       double e1 = 0.0, e2 = 0.0;
@@ -1206,17 +1325,22 @@ SMPC_HD void qs_step(const smpc_problem_t& P, const QsBufs& q, int tile, int lan
       side(QNR + 15 + p, -1.0, azg[5 + p], adg[5 + p], ghi[5 + p], gl[6 + p], gt[6 + p], gp[6 + p], e1, e2);
       if (mode == 0) {
 #pragma unroll
-        for (int c = 0; c < 5; ++c) { const double jv = QF(rec, SMPC_REC_JDIST + p * 5 + c); v1[5 + c] += jv * e1; v2[5 + c] += jv * e2; }
+        for (int c = 0; c < 5; ++c) { const double jv = src.rec(13, SMPC_REC_JDIST + p * 5 + c); v1[5 + c] += jv * e1; v2[5 + c] += jv * e2; }
       }
     }
+  } else {
+    src.release(12);
+    src.acquire(13);
   }
+  src.release(13);
+  src.acquire(14);
   if (F.nn) {
     const double az = azg[11], adz = adg[11];
-    const double v = QF(rec, SMPC_REC_NN);
+    const double v = src.rec(14, SMPC_REC_NN);
     double e1 = 0.0, e2 = 0.0;
     if (!F.soft) {
-      const double l0 = QF(it, I_LAM + 21), t0 = QF(it, I_T + 21), p0 = mode == 1 ? QF(prod, 21) : 0.0;
-      const double l1 = QF(it, I_LAM + QNR + 21), t1 = QF(it, I_T + QNR + 21), p1 = mode == 1 ? QF(prod, QNR + 21) : 0.0;
+      const double l0 = src.it(14, I_LAM + 21), t0 = src.it(14, I_T + 21), p0 = mode == 1 ? src.prod(14, 21) : 0.0;
+      const double l1 = src.it(14, I_LAM + QNR + 21), t1 = src.it(14, I_T + QNR + 21), p1 = mode == 1 ? src.prod(14, QNR + 21) : 0.0;
       side(21, 1.0, az, adz, 0.0 - v, l0, t0, p0, e1, e2);
       side(QNR + 21, -1.0, az, adz, 1e6 - v, l1, t1, p1, e1, e2);
       if (mode != 0) {
@@ -1228,10 +1352,10 @@ SMPC_HD void qs_step(const smpc_problem_t& P, const QsBufs& q, int tile, int lan
       for (int h = 0; h < 2; ++h) {
         const int slot = h * QNR + 21;
         const double sgn = h ? -1.0 : 1.0, bnd = h ? 1e6 - v : 0.0 - v;
-        const double lam = QF(it, I_LAM + slot), t = QF(it, I_T + slot);
-        const double sl = QF(it, I_SLK + h), ls = QF(it, I_SLK + 2 + h), ts = QF(it, I_SLK + 4 + h);
+        const double lam = src.it(14, I_LAM + slot), t = src.it(14, I_T + slot);
+        const double sl = src.it(14, I_SLK + h), ls = src.it(14, I_SLK + 2 + h), ts = src.it(14, I_SLK + 4 + h);
         const double r = t - (sgn * (az - bnd) + sl);
-        const double pr = mode == 1 ? QF(prod, slot) : 0.0, spr = mode == 1 ? QF(prod, 44 + h) : 0.0;
+        const double pr = mode == 1 ? src.prod(14, slot) : 0.0, spr = mode == 1 ? src.prod(14, 44 + h) : 0.0;
         const double rm = qs_rm(mode, lam * t, pr, sigmu);
         const double it_ = 1.0 / t;
         const double G = lam * it_;
@@ -1267,9 +1391,10 @@ SMPC_HD void qs_step(const smpc_problem_t& P, const QsBufs& q, int tile, int lan
     }
     if (mode == 0) {
 #pragma unroll
-      for (int c = 0; c < 10; ++c) { const double jv = QF(rec, SMPC_REC_JNN + c); v1[5 + c] += jv * e1; v2[5 + c] += jv * e2; }
+      for (int c = 0; c < 10; ++c) { const double jv = src.rec(14, SMPC_REC_JNN + c); v1[5 + c] += jv * e1; v2[5 + c] += jv * e2; }
     }
   }
+  src.release(14);
   if (mode == 0) {
     qs_real* vv = q.sb + qs_blk(tile, N, k, NV, lane);
     if (k == N) {
@@ -1281,10 +1406,11 @@ SMPC_HD void qs_step(const smpc_problem_t& P, const QsBufs& q, int tile, int lan
   }
   if (mode == 2) {
     // (dz, dpi) of the step block <- centering direction (after every load of this thread, see the note on load / store phases)
-    const qs_real* st2 = q.st2 + qs_blk(tile, N, k, NS2, lane);
     double dpi[10];
+    src.acquire(15);
 #pragma unroll
-    for (int j = 0; j < 10; ++j) dpi[j] = QF(st2, I_PIM + j);
+    for (int j = 0; j < 10; ++j) dpi[j] = src.st2(15, I_PIM + j);
+    src.release(15);
 #pragma unroll
     for (int i = 0; i < 15; ++i) QF(st, I_Z + i) = dz[i];
 #pragma unroll
@@ -1292,6 +1418,10 @@ SMPC_HD void qs_step(const smpc_problem_t& P, const QsBufs& q, int tile, int lan
   }
   double* stp = q.stp + qs_blk(tile, N, k, NSTP, lane);
   QF(stp, S_ALPHA) = an / ad; QF(stp, S_LIN) = s_lin; QF(stp, S_QUAD) = s_quad;
+}
+SMPC_HD void qs_step(const smpc_problem_t& P, const QsBufs& q, int tile, int lane, int k, int kk, int mode) {
+  QsStepGlobal src(q, tile, lane, k, kk);
+  qs_step(P, q, tile, lane, k, kk, mode, src);
 }
 
 // ================================================================================================================
