@@ -301,7 +301,10 @@ void* smpc_stream(smpc_handle_t* h);
 /* make the handle launch on the caller's stream (cudaStream_t as void*; it must belong to the handle's device and outlive the
  * handle or the next smpc_set_stream) -- what a per-call cudaStream_t argument would do (SURVEY.md section 8(b)), set once instead of
  * passed to every function.  NULL: back to a private non-blocking stream.  Returns after the work queued so far has finished.
- * The legacy default stream is not supported (the QP solver orders its internal streams with events against this one). */
+ * The legacy default stream is not supported (the QP solver orders its internal streams with events against this one).
+ * CUDA graphs: while this stream is being captured, smpc_rti_solve, smpc_controller_step, smpc_plant_step and smpc_sim_step are captured
+ * with their whole QP loop (a conditional WHILE node; the backup solve of smpc_sim_step in a conditional IF node; device pointers only,
+ * not the parallel controller, no profiling; INTEGRATION.md section 3). */
 int smpc_set_stream(smpc_handle_t* h, void* stream);
 int smpc_sync(smpc_handle_t* h);
 

@@ -71,6 +71,7 @@ struct smpc_sim {
   int32_t* outcome_tmp = nullptr;
   unsigned long long* h_requests = nullptr;   // pinned: backup requests so far (SimDev::counters[4])
   unsigned long long requests_seen = 0;
+  cudaStream_t body = nullptr;      // captures the body of the conditional backup solve of a captured step
   std::vector<void*> allocs;        // device buffers of this closed loop (freed by smpc_sim_destroy)
   int device = 0;
 };
@@ -204,6 +205,43 @@ int step_pipeline(smpc_handle* h, const double* x_dev, const uint8_t* act, doubl
   launch_ctrl_post2(c, h->dP, B, N, act, h->xg, h->ug, h->xt, h->ut, h->fails, h->r, h->cur_step, h->need_scan, h->scan11, abort_dev, u_dev);
   if (h->timed) cudaEventRecord(h->ev[3], h->stream);
   return check_launch(h, "controller step pipeline");
+}
+
+// Stream capture (CUDA graphs, INTEGRATION.md).  *cap: the handle's stream is being captured.  A capture that has been invalidated is an
+// error; a captured call must not read anything back on the host, so host arrays, the parallel controller (its early stop reads a
+// counter), profiling / SMPC_QP_TRACE (timelines read on the host) and several tile groups are refused before anything is queued.
+int capture_state(smpc_handle* h, const char* what, bool* cap) {
+  cudaStreamCaptureStatus cs = cudaStreamCaptureStatusNone;
+  const cudaError_t e = cudaStreamIsCapturing(h->stream, &cs);
+  if (e != cudaSuccess) return fail(h, SMPC_ERR_CUDA, what, e);
+  if (cs == cudaStreamCaptureStatusInvalidated) {
+    char buf[256];
+    snprintf(buf, sizeof buf, "%s: the capture of the handle's stream has been invalidated", what);
+    return fail(h, SMPC_ERR_CUDA, buf);
+  }
+  *cap = cs == cudaStreamCaptureStatusActive;
+  return 0;
+}
+int capture_refuse(smpc_handle* h, const char* what, int mem, bool solves) {
+  char buf[256];
+  if (mem == SMPC_HOST) {
+    snprintf(buf, sizeof buf, "%s: host arrays cannot be used in a stream capture (they need a synchronising copy); pass device pointers", what);
+    return fail(h, SMPC_ERR_ARG, buf);
+  }
+  if (!solves) return 0;
+  if (h->P.controller == SMPC_CTRL_PARALLEL) {
+    snprintf(buf, sizeof buf, "%s: the parallel controller cannot be captured (its early stop reads a device counter on the host)", what);
+    return fail(h, SMPC_ERR_UNSUPPORTED, buf);
+  }
+  if (QPCALL(h, qp_traced)) {
+    snprintf(buf, sizeof buf, "%s: profiling / SMPC_QP_TRACE read the kernel timeline on the host and cannot be captured", what);
+    return fail(h, SMPC_ERR_UNSUPPORTED, buf);
+  }
+  if (QPCALL(h, qp_groups) != 1) {
+    snprintf(buf, sizeof buf, "%s: a QP solve over several tile groups (SMPC_QP_GROUPS) cannot be captured", what);
+    return fail(h, SMPC_ERR_UNSUPPORTED, buf);
+  }
+  return 0;
 }
 
 void collect_times(smpc_handle* h, bool with_post) {
@@ -407,22 +445,30 @@ int smpc_reset_controller(smpc_handle_t* h) {
 
 int smpc_rti_solve(smpc_handle_t* h, const double* x0, const uint8_t* active, int32_t* status, int32_t mem) {
   if (!x0) return fail(h, SMPC_ERR_ARG, "smpc_rti_solve: x0 is NULL");
+  bool cap = false;
+  int rc = capture_state(h, "smpc_rti_solve", &cap);
+  if (!rc && cap) rc = capture_refuse(h, "smpc_rti_solve", mem, true);
+  if (rc) return rc;
   const uint8_t* act = nullptr;
-  int rc = mask_in(h, active, mem, &act);
+  rc = mask_in(h, active, mem, &act);
   if (rc) return rc;
   const double* xd = x0;
   if (mem == SMPC_HOST) { rc = copy_in(h, h->x_in, x0, sizeof(double) * h->B * NX, mem); if (rc) return rc; xd = h->x_in; }
-  h->timed = true;
+  h->timed = !cap;                   // (a replay of a captured step records no times: smpc_get_times keeps the last eager step)
   rc = solve_pipeline(h, xd, act);
   if (rc) return rc;
-  h->times_pending = 1;
+  if (!cap) h->times_pending = 1;
   return copy_out(h, status, h->status, sizeof(int32_t) * h->B, mem);
 }
 
 int smpc_controller_step(smpc_handle_t* h, const double* x, const uint8_t* active, double* u, uint8_t* abort_flag, int32_t mem) {
   if (!x || !u) return fail(h, SMPC_ERR_ARG, "smpc_controller_step: x or u is NULL");
+  bool cap = false;
+  int rc = capture_state(h, "smpc_controller_step", &cap);
+  if (!rc && cap) rc = capture_refuse(h, "smpc_controller_step", mem, true);
+  if (rc) return rc;
   const uint8_t* act = nullptr;
-  int rc = mask_in(h, active, mem, &act);
+  rc = mask_in(h, active, mem, &act);
   if (rc) return rc;
   const double* xd = x;
   double* ud = u;
@@ -432,10 +478,10 @@ int smpc_controller_step(smpc_handle_t* h, const double* x, const uint8_t* activ
     rc = copy_in(h, h->u_out, u, sizeof(double) * h->B * NU, mem); if (rc) return rc;   // inactive problems keep the caller's values
     xd = h->x_in; ud = h->u_out; ad = h->abort_flag;
   } else if (!ad) ad = h->abort_flag;
-  h->timed = true;
+  h->timed = !cap;
   rc = step_pipeline(h, xd, act, ud, ad);
   if (rc) return rc;
-  h->times_pending = 2;
+  if (!cap) h->times_pending = 2;
   if (mem == SMPC_HOST) {
     rc = copy_out(h, u, h->u_out, sizeof(double) * h->B * NU, mem); if (rc) return rc;
     rc = copy_out(h, abort_flag, h->abort_flag, (size_t)h->B, mem);
@@ -445,6 +491,10 @@ int smpc_controller_step(smpc_handle_t* h, const double* x, const uint8_t* activ
 
 int smpc_plant_step(smpc_handle_t* h, const double* x, const double* u, double* xn, double* a, int32_t mem) {
   const size_t bx = sizeof(double) * h->B * NX, bu = sizeof(double) * h->B * NU;
+  bool cap = false;
+  int rc0 = capture_state(h, "smpc_plant_step", &cap);
+  if (!rc0 && cap) rc0 = capture_refuse(h, "smpc_plant_step", mem, false);
+  if (rc0) return rc0;
   if (mem == SMPC_DEVICE) {
     launch_plant(h->ctx(), h->dP, h->B, h->plant_inertial, h->tau_noise, x, u, nullptr, xn, a);
     return check_launch(h, "plant_step");
@@ -634,7 +684,8 @@ int smpc_sim_create(smpc_handle_t* c, smpc_handle_t* bk, int32_t n_steps, smpc_s
   CKS(dalloc(c, &d.mode, (size_t)B)); CKS(dalloc(c, &d.ja, (size_t)B)); CKS(dalloc(c, &d.outcome, (size_t)B));
   CKS(dalloc(c, &d.need_ctrl, (size_t)B)); CKS(dalloc(c, &d.need_backup, (size_t)B)); CKS(dalloc(c, &d.abort_flag, (size_t)B));
   CKS(dalloc(c, &d.live, (size_t)B));
-  CKS(dalloc(c, &d.counters, (size_t)5));
+  CKS(dalloc(c, &d.counters, (size_t)SIM_NCOUNTERS));
+  CKS(cudaStreamCreateWithFlags(&s->body, cudaStreamNonBlocking));
   CKS(cudaMallocHost((void**)&s->h_requests, sizeof(unsigned long long)));
   CKS(dalloc(c, &s->outcome_tmp, (size_t)B));
 #undef CKS
@@ -649,6 +700,7 @@ void smpc_sim_destroy(smpc_sim_t* s) {
   cudaDeviceSynchronize();          // (the handles may already be gone: do not touch them)
   for (void* p : s->allocs) cudaFree(p);
   if (s->h_requests) cudaFreeHost(s->h_requests);
+  if (s->body) cudaStreamDestroy(s->body);
   delete s;
 }
 
@@ -662,7 +714,7 @@ int smpc_sim_reset(smpc_sim_t* s, const double* x_init, int32_t mem) {
   launch_fill_f64(lc, d.ulog, (size_t)B * d.n_steps * NU, nan);
   launch_fill_f64(lc, d.xv_first, (size_t)B * NX, nan);
   launch_fill_i32(lc, d.mode, B, 0); launch_fill_i32(lc, d.ja, B, 0); launch_fill_i32(lc, d.outcome, B, 0);
-  CK(c, cudaMemsetAsync(d.counters, 0, 5 * sizeof(unsigned long long), c->stream));
+  CK(c, cudaMemsetAsync(d.counters, 0, SIM_NCOUNTERS * sizeof(unsigned long long), c->stream));
   s->requests_seen = 0;
   int rc = copy_in(c, d.x, x_init, sizeof(double) * B * NX, mem); if (rc) return rc;
   CK(c, cudaMemcpy2DAsync(d.xlog, sizeof(double) * (d.n_steps + 1) * NX, d.x, sizeof(double) * NX, sizeof(double) * NX, B, cudaMemcpyDeviceToDevice, c->stream));
@@ -670,37 +722,82 @@ int smpc_sim_reset(smpc_sim_t* s, const double* x_init, int32_t mem) {
   return check_launch(c, "sim_reset");
 }
 
+// The backup solve of a captured step: a one-thread kernel sets the condition (some problem asked for a backup solve in this step), and
+// the body of a conditional IF node -- captured on s->body, with the backup handle launching there -- holds the backup pipeline, whose
+// QP solve adds its own WHILE node inside (qp.cu).  The caller's stream continues after the IF node.
+static int captured_backup(smpc_sim* s) {
+  smpc_handle* c = s->c;
+  smpc_handle* bk = s->bk;
+  cudaStreamCaptureStatus cs = cudaStreamCaptureStatusNone;
+  cudaGraph_t graph = nullptr;
+  const cudaGraphNode_t* deps = nullptr;
+  size_t n_deps = 0;
+  cudaGraphConditionalHandle cond = 0;
+  CK(c, cudaStreamGetCaptureInfo(c->stream, &cs, nullptr, &graph, &deps, &n_deps));
+  CK(c, cudaGraphConditionalHandleCreate(&cond, graph, 0, 0));     // (no default: the kernel below sets it on every launch)
+  launch_sim_backup_cond(c->ctx(), s->d, cond);
+  CK(c, cudaGetLastError());
+  CK(c, cudaStreamGetCaptureInfo(c->stream, &cs, nullptr, &graph, &deps, &n_deps));
+  cudaGraphNodeParams np = {};
+  np.type = cudaGraphNodeTypeConditional;
+  np.conditional.handle = cond;
+  np.conditional.type = cudaGraphCondTypeIf;
+  np.conditional.size = 1;
+  cudaGraphNode_t node = nullptr;
+  CK(c, cudaGraphAddNode(&node, graph, deps, n_deps, &np));
+  // (from here on a failure leaves the capture with an incomplete node: the error is returned and the capture must be discarded)
+  CK(c, cudaStreamUpdateCaptureDependencies(c->stream, &node, 1, cudaStreamSetCaptureDependencies));
+  CK(c, cudaStreamBeginCaptureToGraph(s->body, np.conditional.phGraph_out[0], nullptr, nullptr, 0, cudaStreamCaptureModeRelaxed));
+  bk->stream = s->body;
+  int rc = solve_pipeline(bk, c->x_viable, s->d.need_backup);   // safe_ocp.solve(x_viable), one RTI (mpc.py:177)
+  bk->stream = c->stream;
+  cudaGraph_t captured = nullptr;
+  const cudaError_t e = cudaStreamEndCapture(s->body, &captured);   // (the body graph belongs to the node)
+  if (rc) { c->err = bk->err; return rc; }
+  if (e != cudaSuccess) return fail(c, SMPC_ERR_CUDA, "smpc_sim_step: capture of the backup solve", e);
+  return 0;
+}
+
 int smpc_sim_step(smpc_sim_t* s) {
   smpc_handle* c = s->c;
   smpc_handle* bk = s->bk;
   SimDev& d = s->d;
   if (s->j >= d.n_steps) return fail(c, SMPC_ERR_ARG, "smpc_sim_step: past n_steps");
+  bool cap = false;
+  int rc = capture_state(c, "smpc_sim_step", &cap);
+  if (!rc && cap) rc = capture_refuse(c, "smpc_sim_step", SMPC_DEVICE, true);
+  if (!rc && cap && (rc = capture_refuse(bk, "smpc_sim_step (backup controller)", SMPC_DEVICE, true))) c->err = bk->err;
+  if (rc) return rc;
   // both handles launch on the main controller's stream so that the step is one ordered sequence
   LaunchCtx lc = c->ctx();
   cudaStream_t bk_stream = bk->stream;
   bk->stream = c->stream;
-  launch_sim_pre(lc, d, c->dP, s->j);
-  c->timed = true; bk->timed = false;           // the main controller's step is timed (smpc_get_times = controller.getTime(), mpc.py:239)
-  int rc = step_pipeline(c, d.x, d.need_ctrl, d.u_ctrl, d.abort_flag);
-  c->times_pending = 2;
-  if (!rc) {
+  // captured: the step index and the backup decision live on the device (sim_pre / sim_post / sim_backup_cond in kernels.cu)
+  launch_sim_pre(lc, d, c->dP, cap ? -1 : s->j);
+  c->timed = !cap; bk->timed = false;           // the main controller's step is timed (smpc_get_times = controller.getTime(), mpc.py:239)
+  rc = step_pipeline(c, d.x, d.need_ctrl, d.u_ctrl, d.abort_flag);
+  if (!cap) c->times_pending = 2;
+  if (!rc && cap) {
+    launch_sim_mid(lc, d, c->x_viable, bk->xg, bk->ug, c->qp_iter);
+    rc = captured_backup(s);                      // conditional IF node around the backup pipeline
+  } else if (!rc) {
     launch_sim_mid(lc, d, c->x_viable, bk->xg, bk->ug, c->qp_iter);
     // the backup OCP is solved only in a step in which some problem aborted (mpc.py:168-177): one 8-byte read-back decides, instead of
     // an empty linearisation + QP launch sequence in every step (the host has waited for the main solve's counters anyway)
-    CK(c, cudaMemcpyAsync(s->h_requests, d.counters + 4, sizeof(unsigned long long), cudaMemcpyDeviceToHost, c->stream));
-    CK(c, cudaStreamSynchronize(c->stream));
-    if (*s->h_requests != s->requests_seen) {
+    cudaError_t e = cudaMemcpyAsync(s->h_requests, d.counters + 4, sizeof(unsigned long long), cudaMemcpyDeviceToHost, c->stream);
+    if (e == cudaSuccess) e = cudaStreamSynchronize(c->stream);
+    if (e != cudaSuccess) rc = fail(c, SMPC_ERR_CUDA, "smpc_sim_step: backup request read-back", e);
+    else if (*s->h_requests != s->requests_seen) {
       s->requests_seen = *s->h_requests;
       rc = solve_pipeline(bk, c->x_viable, d.need_backup);   // safe_ocp.solve(x_viable), one RTI (mpc.py:177)
     }
   }
   if (!rc) {
-    launch_sim_post(lc, d, c->dP, s->j, bk->status, bk->xt, bk->ut, c->plant_inertial, c->tau_noise, bk->qp_iter);
+    launch_sim_post(lc, d, c->dP, cap ? -1 : s->j, bk->status, bk->xt, bk->ut, c->plant_inertial, c->tau_noise, bk->qp_iter);
     rc = check_launch(c, "sim_step");
   }
-  bk->stream = bk_stream;
-  c->launches += 0;
-  s->j += 1;
+  bk->stream = bk_stream;                        // (restored on every path)
+  if (!cap) s->j += 1;                           // (a captured step advances the device-side index on every replay)
   return rc;
 }
 int smpc_sim_run(smpc_sim_t* s, int32_t n) {

@@ -100,13 +100,19 @@ struct SimDev {
   double *x, *xlog, *ulog, *x_abort, *u_abort, *xv_first, *u_ctrl, *u;
   int32_t *mode, *ja, *outcome;
   uint8_t *need_ctrl, *need_backup, *abort_flag, *live;
-  unsigned long long* counters;   // [5]: RTI solves, backup solves, plant steps, IPM iterations; [4] = backup requests so far (host: skip the empty backup solve)
+  unsigned long long* counters;   // [SIM_NCOUNTERS]: RTI solves, backup solves, plant steps, IPM iterations; [4] = backup requests so far (host: skip the
+                                  // empty backup solve); then the device-side step bookkeeping of captured steps (below)
 };
+enum { SIM_REQ_SEEN = 5,          // backup requests at the start of the current captured step
+       SIM_STEP_CUR = 6,          // index of the current captured step
+       SIM_STEP_NEXT = 7,         // index of the next step (written by every step, eager or captured)
+       SIM_NCOUNTERS = 8 };
 void launch_sim_pre(const LaunchCtx& c, const SimDev& s, const smpc_problem_t* dP, int j);
 void launch_sim_mid(const LaunchCtx& c, const SimDev& s, const double* x_viable, double* bk_xg, double* bk_ug, const int32_t* qp_iter_main);
 void launch_sim_post(const LaunchCtx& c, const SimDev& s, const smpc_problem_t* dP, int j, const int32_t* bk_status, const double* bk_xt,
                      const double* bk_ut, const double* inertial, const double* noise, const int32_t* qp_iter_bk);
 void launch_sim_outcome(const LaunchCtx& c, const SimDev& s, const smpc_problem_t* dP, int32_t* out);
+void launch_sim_backup_cond(const LaunchCtx& c, const SimDev& s, cudaGraphConditionalHandle cond);
 
 // qp.cu -- split interior-point solver (qp_split.cuh).  The library holds it twice: qp.cu (fp64 storage, namespace smpc::f64) and
 // qp_f32.cu (the same source with QS_REAL = float, namespace smpc::f32); the flavour of this translation unit is an inline namespace.
@@ -120,6 +126,7 @@ void launch_sim_outcome(const LaunchCtx& c, const SimDev& s, const smpc_problem_
   int qp_last_iterations(const QpSolver* s);                                                                                              \
   int qp_compactions(const QpSolver* s);   /* compactions of the slots during the last solve (> 0: per-slot dumps are gone) */            \
   void qp_set_profiling(QpSolver* s, bool on);                                                                                            \
+  bool qp_traced(const QpSolver* s);       /* profiling or SMPC_QP_TRACE: the solve reads events back on the host */                      \
   void qp_get_profile(const QpSolver* s, double* ms, int32_t* n, double* span_ms);                                                        \
   /* one batched solve; reads the records of qp_rec(); problems with act == 0 are skipped and keep their outputs */                      \
   cudaError_t launch_qp_solve(const LaunchCtx& c, const smpc_problem_t* dP, QpSolver* s, const double* x0, const int32_t* r,              \

@@ -634,8 +634,11 @@ void launch_set_xviable_from_guess(const LaunchCtx& c, int B, int N, const doubl
 // Closed loop (reference scripts/mpc.py:125-264).  Per problem: mode 0 = MPC, 1 = following the abort trajectory /
 // PD hold, 2 = terminated.
 // ----------------------------------------------------------------------------------------------------------------
+// j < 0: a step captured into a CUDA graph -- the step index comes from the device (SIM_STEP_NEXT, kept by sim_post) and the backup
+// request count at the start of the step is noted for the conditional node that decides on the backup solve (sim_backup_cond_kernel)
 __global__ void sim_pre_kernel(SimDev s, const smpc_problem_t* __restrict__ dP, int j) {
   const int b = blockIdx.x * blockDim.x + threadIdx.x;
+  if (j < 0 && b == 0) { s.counters[SIM_STEP_CUR] = s.counters[SIM_STEP_NEXT]; s.counters[SIM_REQ_SEEN] = s.counters[4]; }
   if (b >= s.B) return;
   const int Nb = s.Nb;
   s.need_ctrl[b] = 0; s.need_backup[b] = 0; s.live[b] = 0;
@@ -700,7 +703,9 @@ __global__ void sim_post_kernel(SimDev s, const smpc_problem_t* __restrict__ dP,
                                 const double* __restrict__ bk_xt, const double* __restrict__ bk_ut, const double* __restrict__ inertial,
                                 const double* __restrict__ noise, const int32_t* __restrict__ qp_iter_bk) {
   const int b = blockIdx.x * blockDim.x + threadIdx.x;
-  if (b >= s.B) return;
+  if (j < 0) j = (int)s.counters[SIM_STEP_CUR];
+  if (b == 0) s.counters[SIM_STEP_NEXT] = (unsigned long long)j + 1;
+  if (b >= s.B || j >= s.n_steps) return;          // (a replay past the end of the log does nothing)
   if (!s.live[b]) return;
   const smpc_problem_t& P = *dP;
   const int Nb = s.Nb;
@@ -748,6 +753,15 @@ __global__ void sim_outcome_kernel(SimDev s, const smpc_problem_t* __restrict__ 
   if (sqrt(d2) < P.tol_conv) o |= SMPC_OUT_CONVERGED;
   out[b] = o;
 }
+// condition of the conditional IF node around the backup solve of a captured step: some problem asked for it in this step
+__global__ void __launch_bounds__(1) sim_backup_cond_kernel(const unsigned long long* __restrict__ counters, cudaGraphConditionalHandle cond) {
+  cudaGraphSetConditional(cond, counters[4] != counters[SIM_REQ_SEEN] ? 1u : 0u);
+}
+void launch_sim_backup_cond(const LaunchCtx& c, const SimDev& s, cudaGraphConditionalHandle cond) {
+  sim_backup_cond_kernel<<<1, 1, 0, c.stream>>>(s.counters, cond);
+  ++*c.launches;
+}
+
 void launch_sim_outcome(const LaunchCtx& c, const SimDev& s, const smpc_problem_t* dP, int32_t* out) {
   sim_outcome_kernel<<<GRID1D(s.B, 128), 128, 0, c.stream>>>(s, dP, out);
   ++*c.launches;

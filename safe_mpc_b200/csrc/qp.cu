@@ -55,7 +55,9 @@ __global__ void __launch_bounds__(32) qs_init_kernel(QsBufs q, int B, const doub
 constexpr size_t PREP_SMEM = sizeof(double) * 2 * PREP_SCRATCH * TL + 512;   // a retiring prep CTA leaves room for one Riccati CTA
 constexpr int PREP_WARPS = 2;    // warps per CTA of prep: 2 x 26.9 KB of lane-private Jacobian scratch, 4 CTAs per SM
 template <bool FIRST>
-__global__ void __launch_bounds__(32 * PREP_WARPS, QS_PREP_MINB) qs_prep_kernel(const smpc_problem_t* __restrict__ dP, QsBufs q, int T, int kk) {
+__global__ void __launch_bounds__(32 * PREP_WARPS, QS_PREP_MINB) qs_prep_kernel(const smpc_problem_t* __restrict__ dP, QsBufs q, int T, int kk,
+                                                                                          const int* __restrict__ kk_dev) {
+  if (kk_dev) kk = *kk_dev;
   extern __shared__ __align__(128) double jsm_all[];
   const int wi = threadIdx.x >> 5;
   const int w = blockIdx.x * PREP_WARPS + wi;
@@ -90,7 +92,9 @@ __device__ __forceinline__ void pc_row_out(double* s_it, int sl, double nu, doub
   QF(s_it, I_LAM + sl) = nu; QF(s_it, I_LAM + QNR + sl) = gam; QF(s_it, I_T + sl) = G;
 }
 
-__global__ void __launch_bounds__(32 * PC_WARPS, 2) qs_prep_coop_kernel(const smpc_problem_t* __restrict__ dP, QsBufs q, int T, int kk) {
+__global__ void __launch_bounds__(32 * PC_WARPS, 2) qs_prep_coop_kernel(const smpc_problem_t* __restrict__ dP, QsBufs q, int T, int kk,
+                                                                      const int* __restrict__ kk_dev) {
+  if (kk_dev) kk = *kk_dev;
   extern __shared__ __align__(128) double pc_sm[];
   const smpc_problem_t& P = *dP;
   const int N = q.N;
@@ -466,7 +470,9 @@ __global__ void __launch_bounds__(32 * PC_WARPS, 2) qs_prep_coop_kernel(const sm
 }
 
 template <int MODE>
-__global__ void __launch_bounds__(32 * SP_WARPS, QS_SP_MINB) qs_step_kernel(const smpc_problem_t* __restrict__ dP, QsBufs q, int T, int kk) {
+__global__ void __launch_bounds__(32 * SP_WARPS, QS_SP_MINB) qs_step_kernel(const smpc_problem_t* __restrict__ dP, QsBufs q, int T, int kk,
+                                                                                  const int* __restrict__ kk_dev) {
+  if (kk_dev) kk = *kk_dev;
   const int w = blockIdx.x * SP_WARPS + (threadIdx.x >> 5);
   if (w >= T * (q.N + 1)) return;
   qs_step(*dP, q, w / (q.N + 1), threadIdx.x & 31, w % (q.N + 1), kk, MODE);
@@ -558,7 +564,9 @@ struct StepRing {
 };
 
 template <int MODE>
-__global__ void __launch_bounds__(32 * SP_WARPS, QS_SP_MINB) qs_step_ring_kernel(const smpc_problem_t* __restrict__ dP, QsBufs q, int T, int kk) {
+__global__ void __launch_bounds__(32 * SP_WARPS, QS_SP_MINB) qs_step_ring_kernel(const smpc_problem_t* __restrict__ dP, QsBufs q, int T, int kk,
+                                                                                       const int* __restrict__ kk_dev) {
+  if (kk_dev) kk = *kk_dev;
   extern __shared__ __align__(128) unsigned char sr_sm[];
   const int wi = threadIdx.x >> 5, lane = threadIdx.x & 31;
   const int w = blockIdx.x * SP_WARPS + wi;
@@ -582,7 +590,8 @@ __global__ void __launch_bounds__(32 * SP_WARPS, QS_SP_MINB) qs_step_ring_kernel
 }
 
 __global__ void __launch_bounds__(32) qs_ctl_kernel(const smpc_problem_t* __restrict__ dP, QsBufs q, int kk, int32_t* status, int32_t* qp_iter,
-                                                     int32_t* qp_status, double* qp_res, int* counters) {
+                                                     int32_t* qp_status, double* qp_res, int* counters, const int* __restrict__ kk_dev) {
+  if (kk_dev) kk = *kk_dev;
   const bool on = qs_ctl<16>(*dP, q, blockIdx.x, threadIdx.x, kk, status, qp_iter, qp_status, qp_res);
   const unsigned m = __ballot_sync(0xffffffffu, on);
   if (threadIdx.x == 0 && m) atomicAdd(&counters[2 * kk], __popc(m));
@@ -1109,7 +1118,9 @@ __global__ void __launch_bounds__(32) qs_ric2_kernel(const smpc_problem_t* __res
 }
 
 // redo_list: the slots (of this group) whose problem fell back to the centering direction, tile by tile in arrival order of the tiles
-__global__ void __launch_bounds__(32) qs_red_kernel(const smpc_problem_t* __restrict__ dP, QsBufs q, int kk, int after_redo, int* counters, int32_t* redo_list) {
+__global__ void __launch_bounds__(32) qs_red_kernel(const smpc_problem_t* __restrict__ dP, QsBufs q, int kk, int after_redo, int* counters, int32_t* redo_list,
+                                                    const int* __restrict__ kk_dev) {
+  if (kk_dev) kk = *kk_dev;
   qs_red(*dP, q, blockIdx.x, threadIdx.x, after_redo != 0);
   if (!after_redo) {
     const int32_t* pi = q.pi + qs_pb(blockIdx.x, NPI, threadIdx.x);
@@ -1120,6 +1131,17 @@ __global__ void __launch_bounds__(32) qs_red_kernel(const smpc_problem_t* __rest
     base = __shfl_sync(0xffffffffu, base, 0);
     if (redo) redo_list[base + __popc(m & ((1u << threadIdx.x) - 1u))] = blockIdx.x * TL + threadIdx.x;
   }
+}
+
+// Device-side loop of a solve captured into a CUDA graph (qp_split.cuh: qs_graph_drive), one thread each.  reset: every launch of the
+// graph starts a fresh solve at iteration 0 and enters the loop body;  loop: the loop step of qs_loop_step sets the condition of the
+// WHILE node that repeats the body.
+__global__ void __launch_bounds__(1) qs_loop_reset_kernel(int* kk_dev, cudaGraphConditionalHandle cond) {
+  *kk_dev = 0;
+  cudaGraphSetConditional(cond, 1);
+}
+__global__ void __launch_bounds__(1) qs_loop_kernel(const int* __restrict__ counters, int* kk_dev, int iter_max, cudaGraphConditionalHandle cond) {
+  cudaGraphSetConditional(cond, qs_loop_step(counters, kk_dev, iter_max) ? 1u : 0u);
 }
 
 // The switch to the centering direction for FEW flagged problems: one CTA per list entry, thread = stage (qs_step mode 2), then thread 0
@@ -1205,6 +1227,8 @@ struct QpGroup {
   int* n_moves = nullptr;       // device
   int32_t* redo_list = nullptr; // [32 T] slots flagged for the centering direction in the current iteration (qs_red_kernel)
   int in_use = 0;               // slots that may still hold an iterating problem (32 T at the start of a solve, less after a compaction)
+  int* kk_dev = nullptr;        // IPM iteration of a solve captured into a graph (device)
+  cudaStream_t body = nullptr;  // captures the loop body of such a solve
   int tiles() const { return (in_use + TL - 1) / TL; }
 };
 
@@ -1216,6 +1240,7 @@ struct QpSolver {
   int32_t* pi = nullptr;
   int* counters = nullptr;
   int* h_counters = nullptr;
+  int* kk_dev = nullptr;        // [G]
   int32_t* mv = nullptr;        // compaction plans of the groups
   int* n_moves = nullptr;
   int32_t* redo_list = nullptr;
@@ -1272,6 +1297,7 @@ QpSolver* qp_create(int B, int N, int iter_max, bool keep_slots, cudaStream_t st
   if (e == cudaSuccess) e = cudaMemsetAsync(s->pi, 0, sizeof(int32_t) * T * NPI * TL, stream);
   if (e == cudaSuccess) e = cudaMalloc((void**)&s->counters, sizeof(int) * ncnt * G);
   if (e == cudaSuccess) e = cudaMallocHost((void**)&s->h_counters, sizeof(int) * 2 * RING * G);
+  if (e == cudaSuccess) e = cudaMalloc((void**)&s->kk_dev, sizeof(int) * G);
   if (e == cudaSuccess) e = cudaEventCreateWithFlags(&s->ev_in, cudaEventDisableTiming);
   if (e == cudaSuccess) e = cudaMalloc((void**)&s->mv, sizeof(int32_t) * ((size_t)s->T * TL + 2 * MAX_GROUPS));
   if (e == cudaSuccess) e = cudaMalloc((void**)&s->n_moves, sizeof(int) * MAX_GROUPS);
@@ -1311,6 +1337,7 @@ QpSolver* qp_create(int B, int N, int iter_max, bool keep_slots, cudaStream_t st
     for (int i = 0; i < RING && e == cudaSuccess; ++i) e = cudaEventCreateWithFlags(&s->grp[g].ev[i], cudaEventDisableTiming);
     if (e == cudaSuccess) e = cudaEventCreateWithFlags(&s->grp[g].ev_done, cudaEventDisableTiming);
     if (e == cudaSuccess) e = cudaEventCreateWithFlags(&s->grp[g].evx, cudaEventDisableTiming);
+    if (e == cudaSuccess) e = cudaStreamCreateWithFlags(&s->grp[g].body, cudaStreamNonBlocking);
   }
   if (e != cudaSuccess) { *err = e; qp_destroy(s); return nullptr; }
   double* p = s->block;
@@ -1345,6 +1372,7 @@ QpSolver* qp_create(int B, int N, int iter_max, bool keep_slots, cudaStream_t st
     gr.n_moves = s->n_moves + g;
     gr.redo_list = s->redo_list + (size_t)t0 * TL;
     gr.in_use = gr.T * TL;
+    gr.kk_dev = s->kk_dev + g;
   }
   *err = cudaSuccess;
   return s;
@@ -1358,11 +1386,13 @@ void qp_destroy(QpSolver* s) {
     for (int i = 0; i < RING; ++i) if (s->grp[g].ev[i]) cudaEventDestroy(s->grp[g].ev[i]);
     if (s->grp[g].ev_done) cudaEventDestroy(s->grp[g].ev_done);
     if (s->grp[g].evx) cudaEventDestroy(s->grp[g].evx);
+    if (s->grp[g].body) cudaStreamDestroy(s->grp[g].body);
   }
   if (s->ev_in) cudaEventDestroy(s->ev_in);
   if (s->block) cudaFree(s->block);
   if (s->pi) cudaFree(s->pi);
   if (s->counters) cudaFree(s->counters);
+  if (s->kk_dev) cudaFree(s->kk_dev);
   if (s->h_counters) cudaFreeHost(s->h_counters);
   if (s->mv) cudaFree(s->mv);
   if (s->n_moves) cudaFree(s->n_moves);
@@ -1375,6 +1405,7 @@ int qp_last_iterations(const QpSolver* s) { return s->last_iters; }
 int qp_groups(const QpSolver* s) { return s->G; }
 int qp_compactions(const QpSolver* s) { return s->n_compactions; }
 void qp_set_profiling(QpSolver* s, bool on) { s->profile = on; }
+bool qp_traced(const QpSolver* s) { return s->profile || s->trace_print; }
 void qp_get_profile(const QpSolver* s, double* ms, int32_t* n, double* span_ms) {
   for (int i = 0; i < SMPC_PROF_N; ++i) { ms[i] = s->prof_ms[i]; n[i] = s->prof_n[i]; }
   *span_ms = s->prof_span_ms;
@@ -1403,9 +1434,16 @@ struct DeviceBackend {
   bool red_done = false;        // the list form of the centering switch has already taken the step length: the next red(true) is a no-op
   cudaError_t err = cudaSuccess;
   bool on_hi = false;
+  // solve captured into a CUDA graph (qs_graph_drive): no host reads; while the loop body is being captured, every kernel goes to the
+  // body stream and takes its iteration from g->kk_dev, in the fixed forms of DESIGN §3.2
+  bool graph = false;
+  cudaStream_t in_body = nullptr;
+  cudaGraphConditionalHandle cond = 0;
+  const int* kd() const { return in_body ? g->kk_dev : nullptr; }
   bool trace_on() const { return s->profile || s->trace_print; }
   // stream for the next kernel; a change of stream is ordered after everything queued on the other one
   cudaStream_t st(bool hi) {
+    if (in_body) return in_body;
     if (!g->hi) return g->stream;
     if (hi != on_hi) {
       cudaEventRecord(g->evx, on_hi ? g->hi : g->stream);
@@ -1430,7 +1468,9 @@ struct DeviceBackend {
   void tr1(cudaStream_t stm) { if (trace_on()) cudaEventRecord(s->trace.back().b, stm); }
   void init() {
     g->in_use = g->T * TL;
-    cudaMemsetAsync(g->counters, 0, sizeof(int) * 2 * (s->iter_max + 2), st(false));
+    // (a captured solve may end up inside a conditional body, which takes kernel nodes only)
+    if (graph) { launch_fill_i32(LaunchCtx{st(false), launches}, g->counters, 2 * (s->iter_max + 2), 0); }
+    else cudaMemsetAsync(g->counters, 0, sizeof(int) * 2 * (s->iter_max + 2), st(false));
     { cudaStream_t stm_ = st(false); tr0("qs_init_kernel", stm_); qs_init_kernel<<<g->T, 32, 0, stm_>>>(g->q, s->B, x0, r, act); tr1(stm_); }
     count();
   }
@@ -1439,26 +1479,27 @@ struct DeviceBackend {
       cudaStream_t stm_ = st(false);
       const int grid = (tl() * (s->N + 1) + PREP_WARPS - 1) / PREP_WARPS;
       tr0("qs_prep_kernel", stm_);
-      if (kk == 0) qs_prep_kernel<true><<<grid, 32 * PREP_WARPS, PREP_SMEM, stm_>>>(dP, g->q, tl(), kk);
+      if (kk == 0 && !in_body) qs_prep_kernel<true><<<grid, 32 * PREP_WARPS, PREP_SMEM, stm_>>>(dP, g->q, tl(), kk, nullptr);
       // the cooperative form stages whole (tile, stage) blocks, the thread-per-stage form only touches the lanes that still iterate:
       // measured break-even at about half of the slots in use active (full launch 0.57 ms against 1.02 ms).  In the deep tail (a handful
       // of tiles) throughput does not matter and the cooperative form has the shorter critical path (33 against 43 us)
-      else if (s->coop_prep && (2 * n_active_last >= g->in_use || n_active_last <= s->tail_max)) qs_prep_coop_kernel<<<tl() * (s->N + 1), 32 * PC_WARPS, PC_SMEM, stm_>>>(dP, g->q, tl(), kk);
-      else qs_prep_kernel<false><<<grid, 32 * PREP_WARPS, PREP_SMEM, stm_>>>(dP, g->q, tl(), kk);
+      else if (s->coop_prep && (in_body || 2 * n_active_last >= g->in_use || n_active_last <= s->tail_max))
+        qs_prep_coop_kernel<<<tl() * (s->N + 1), 32 * PC_WARPS, PC_SMEM, stm_>>>(dP, g->q, tl(), kk, kd());
+      else qs_prep_kernel<false><<<grid, 32 * PREP_WARPS, PREP_SMEM, stm_>>>(dP, g->q, tl(), kk, kd());
       tr1(stm_);
     }
     count();
   }
   void ctl(int kk) {
     kk_last = kk;
-    { cudaStream_t stm_ = st(false); tr0("qs_ctl_kernel", stm_); qs_ctl_kernel<<<tl(), 32, 0, stm_>>>(dP, g->q, kk, status, qp_iter, qp_status, qp_res, g->counters); tr1(stm_); }
+    { cudaStream_t stm_ = st(false); tr0("qs_ctl_kernel", stm_); qs_ctl_kernel<<<tl(), 32, 0, stm_>>>(dP, g->q, kk, status, qp_iter, qp_status, qp_res, g->counters, kd()); tr1(stm_); }
     count();
   }
   void ric1() {
     {
       cudaStream_t stm_ = st(true);
       tr0("qs_ric1_kernel", stm_);
-      if (n_active_last <= s->tail_max && (s->tail_which & 1)) qs_ric1t_kernel<<<tl() * (32 / RT_WARPS), 32 * RT_WARPS, RT_SMEM, stm_>>>(dP, g->q);
+      if (!in_body && n_active_last <= s->tail_max && (s->tail_which & 1)) qs_ric1t_kernel<<<tl() * (32 / RT_WARPS), 32 * RT_WARPS, RT_SMEM, stm_>>>(dP, g->q);
       else if (s->split_ric1) qs_ric1x_kernel<<<tl(), 64, RIC1X_SMEM, stm_>>>(dP, g->q);
       else qs_ric1_kernel<<<tl(), 32, RIC1_SMEM, stm_>>>(dP, g->q);
       tr1(stm_);
@@ -1469,7 +1510,7 @@ struct DeviceBackend {
     {
       cudaStream_t stm_ = st(true);
       tr0("qs_ric2_kernel", stm_);
-      if (n_active_last <= s->tail_max && (s->tail_which & 2)) qs_ric2t_kernel<<<tl() * (32 / RT_WARPS), 32 * RT_WARPS, RT_SMEM, stm_>>>(dP, g->q);
+      if (!in_body && n_active_last <= s->tail_max && (s->tail_which & 2)) qs_ric2t_kernel<<<tl() * (32 / RT_WARPS), 32 * RT_WARPS, RT_SMEM, stm_>>>(dP, g->q);
       else qs_ric2_kernel<<<tl(), 32, RIC2_SMEM, stm_>>>(dP, g->q);
       tr1(stm_);
     }
@@ -1477,8 +1518,8 @@ struct DeviceBackend {
   }
   template <int MODE>
   void step_pass(cudaStream_t stm_, int kk, bool ring) {
-    if (ring) qs_step_ring_kernel<MODE><<<sp_grid(), 32 * SP_WARPS, SR_SMEM, stm_>>>(dP, g->q, tl(), kk);
-    else qs_step_kernel<MODE><<<sp_grid(), 32 * SP_WARPS, 0, stm_>>>(dP, g->q, tl(), kk);
+    if (ring) qs_step_ring_kernel<MODE><<<sp_grid(), 32 * SP_WARPS, SR_SMEM, stm_>>>(dP, g->q, tl(), kk, kd());
+    else qs_step_kernel<MODE><<<sp_grid(), 32 * SP_WARPS, 0, stm_>>>(dP, g->q, tl(), kk, kd());
   }
   void step(int kk, int mode) {
     if (mode == 0) { cudaStream_t stm_ = st(false); tr0("qs_step_kernel<0>", stm_); step_pass<0>(stm_, kk, s->ring_step); tr1(stm_); }
@@ -1488,7 +1529,7 @@ struct DeviceBackend {
       tr0("qs_step_kernel<2>", stm_);
       // (the host knows the number of flagged problems only when it has waited for the counters of THIS iteration: depth 0)
       const int lim = s->redo_list_max < 0 ? g->in_use / 8 : s->redo_list_max;
-      if (n_redo_kk == kk && n_redo_last > 0 && n_redo_last <= lim) {
+      if (!in_body && n_redo_kk == kk && n_redo_last > 0 && n_redo_last <= lim) {
         qs_redo_list_kernel<<<n_redo_last, RL_THREADS, 0, stm_>>>(dP, g->q, kk, g->redo_list, g->counters + 2 * kk + 1);
         red_done = true;
       } else step_pass<2>(stm_, kk, s->ring_step);
@@ -1512,7 +1553,7 @@ struct DeviceBackend {
   void final() { { cudaStream_t stm_ = st(false); tr0("qs_final_kernel", stm_); qs_final_kernel<<<sp_grid_all(), 32 * SP_WARPS, 0, stm_>>>(g->q, g->T, s->B, act, status, xt, ut); tr1(stm_); } count(); }
   void red(bool after) {
     if (after && red_done) { red_done = false; return; }
-    { cudaStream_t stm_ = st(false); tr0("qs_red_kernel", stm_); qs_red_kernel<<<tl(), 32, 0, stm_>>>(dP, g->q, kk_last, after ? 1 : 0, g->counters, g->redo_list); tr1(stm_); }
+    { cudaStream_t stm_ = st(false); tr0("qs_red_kernel", stm_); qs_red_kernel<<<tl(), 32, 0, stm_>>>(dP, g->q, kk_last, after ? 1 : 0, g->counters, g->redo_list, kd()); tr1(stm_); }
     count();
   }
   // Compaction between iteration kk and kk + 1 (qp_split.cuh: qs_compact_*), decided on the newest active count the host has seen --
@@ -1537,6 +1578,47 @@ struct DeviceBackend {
     g->in_use = na;
     s->compacted = true;
     s->n_compactions += 1;
+  }
+  // Device-side loop (qs_graph_drive): a reset kernel, then a conditional WHILE node whose body graph is captured on g->body by one
+  // call of body(*this); the node joins the capture of the group stream, and the kernels queued after loop() follow it
+  template <class F>
+  void loop(F body) {
+    cudaStream_t stm_ = st(false);
+    cudaStreamCaptureStatus cs = cudaStreamCaptureStatusNone;
+    cudaGraph_t graph = nullptr;
+    const cudaGraphNode_t* deps = nullptr;
+    size_t n_deps = 0;
+    cudaError_t e = cudaStreamGetCaptureInfo(stm_, &cs, nullptr, &graph, &deps, &n_deps);
+    if (e == cudaSuccess && cs != cudaStreamCaptureStatusActive) e = cudaErrorStreamCaptureInvalidated;
+    if (e == cudaSuccess) e = cudaGraphConditionalHandleCreate(&cond, graph, 1, cudaGraphCondAssignDefault);
+    if (e == cudaSuccess) {
+      qs_loop_reset_kernel<<<1, 1, 0, stm_>>>(g->kk_dev, cond);
+      count();
+      e = cudaStreamGetCaptureInfo(stm_, &cs, nullptr, &graph, &deps, &n_deps);
+    }
+    cudaGraphNodeParams np = {};
+    np.type = cudaGraphNodeTypeConditional;
+    np.conditional.handle = cond;
+    np.conditional.type = cudaGraphCondTypeWhile;
+    np.conditional.size = 1;
+    cudaGraphNode_t node = nullptr;
+    if (e == cudaSuccess) e = cudaGraphAddNode(&node, graph, deps, n_deps, &np);
+    // (a failure past this point leaves the capture holding a WHILE node with an empty body; the error is returned and the caller has to
+    // discard the capture)
+    if (e == cudaSuccess) e = cudaStreamUpdateCaptureDependencies(stm_, &node, 1, cudaStreamSetCaptureDependencies);
+    if (e == cudaSuccess) e = cudaStreamBeginCaptureToGraph(g->body, np.conditional.phGraph_out[0], nullptr, nullptr, 0, cudaStreamCaptureModeRelaxed);
+    if (e != cudaSuccess) { err = e; return; }
+    in_body = g->body;
+    body(*this);
+    in_body = nullptr;
+    cudaGraph_t captured = nullptr;
+    e = cudaStreamEndCapture(g->body, &captured);     // (the body graph belongs to the node)
+    if (e != cudaSuccess && err == cudaSuccess) err = e;
+  }
+  void loop_step() {
+    cudaStream_t stm_ = st(false);
+    qs_loop_kernel<<<1, 1, 0, stm_>>>(g->counters, g->kk_dev, s->iter_max, cond);
+    count();
   }
   void request_counters(int kk) {
     const int slot = kk % RING;
@@ -1568,14 +1650,29 @@ struct DeviceBackend {
 cudaError_t launch_qp_solve(const LaunchCtx& c, const smpc_problem_t* dP, QpSolver* s, const double* x0, const int32_t* r, const uint8_t* act,
                             double* xt, double* ut, int32_t* status, int32_t* qp_iter, int32_t* qp_status, double* qp_res) {
   s->compacted = false; s->n_compactions = 0;
+  // a solve captured into a CUDA graph runs its loop on the device (one tile group, no host-side timeline; api.cu refuses the rest
+  // before anything is queued)
+  cudaStreamCaptureStatus cs = cudaStreamCaptureStatusNone;
+  cudaError_t e = cudaStreamIsCapturing(c.stream, &cs);
+  if (e != cudaSuccess) return e;
+  const bool graph = cs == cudaStreamCaptureStatusActive;
+  if (graph && (s->G != 1 || s->profile || s->trace_print)) return cudaErrorNotSupported;
   // the group streams start after everything queued on the caller's stream (linearisation, input copies) ...
-  cudaError_t e = cudaEventRecord(s->ev_in, c.stream);
+  e = cudaEventRecord(s->ev_in, c.stream);
   if (e != cudaSuccess) return e;
   DeviceBackend bk[MAX_GROUPS];
   for (int g = 0; g < s->G; ++g) {
     e = cudaStreamWaitEvent(s->grp[g].stream, s->ev_in, 0);
     if (e != cudaSuccess) return e;
     bk[g] = DeviceBackend{c.launches, dP, s, &s->grp[g], x0, r, act, xt, ut, status, qp_iter, qp_status, qp_res};
+  }
+  if (graph) {
+    bk[0].graph = true;
+    qs_graph_drive(bk[0]);
+    if (bk[0].err != cudaSuccess) return bk[0].err;
+    e = cudaEventRecord(s->grp[0].ev_done, bk[0].st(false));
+    if (e == cudaSuccess) e = cudaStreamWaitEvent(c.stream, s->grp[0].ev_done, 0);
+    return e;
   }
   s->last_iters = qs_drive(bk, s->G, s->depth);
   if (s->profile || s->trace_print) {

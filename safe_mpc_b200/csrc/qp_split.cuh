@@ -1527,5 +1527,40 @@ int qs_drive(BK* groups, int n_groups, int depth = 0) {
   return kmax;
 }
 
+// Device-side sequencing of one solve (a solve captured into a CUDA graph: the host cannot read counters, DESIGN §3.2).  The
+// iteration index lives in device memory (*kk); one iteration is the run-ahead order of QsLoop::issue with step<2> / red queued
+// unconditionally, followed by the loop step below and the prep of the next iterate.  The backend repeats the body while the loop
+// step says so: qp.cu as a conditional WHILE node of the graph, tests/graph_loop_host.cpp as a plain loop.
+// Loop step (one thread): reads the active count of iteration *kk, advances *kk, and returns whether the body runs again.
+SMPC_HD bool qs_loop_continue(int n_active, int kk, int iter_max) { return n_active > 0 && kk < iter_max; }
+SMPC_HD bool qs_loop_step(const int* counters, int* kk, int iter_max) {
+  const int k = *kk;
+  *kk = k + 1;
+  return qs_loop_continue(counters[2 * k], k, iter_max);
+}
+
+template <class BK>
+void qs_graph_body(BK& bk) {
+  bk.ctl(0);
+  bk.ric1();
+  bk.step(0, 0);
+  bk.ric2();
+  bk.step(0, 1);
+  bk.red(false);
+  bk.step(0, 2);
+  bk.red(true);
+  bk.loop_step();
+  bk.prep(0);          // the iterate of the new *kk
+}
+
+// init and prep(0) as in QsLoop::start; the solo kernel when the backend takes it (decided from what the host knows at iteration 0),
+// else the device-side loop; then final
+template <class BK>
+void qs_graph_drive(BK& bk) {
+  bk.init(); bk.prep(0);
+  if (!bk.solo(0)) bk.loop(qs_graph_body<BK>);
+  bk.final();
+}
+
 }  // inline namespace QS_FLAVOUR
 }  // namespace smpc
